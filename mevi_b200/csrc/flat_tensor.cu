@@ -150,11 +150,22 @@ __global__ void flat_consts_kernel(const unsigned* docmeta, const unsigned* absm
   }
 }
 
-// per-query slack: a true top-k member's approximate score is at least (k-th approximate) - 2 E_max
-__global__ void flat_margin_kernel(const float* __restrict__ qnorm, int nq, const unsigned* __restrict__ dmax_bits,
-                                   float* __restrict__ margin) {
+// per-query slack: a true top-k member's approximate score is at least (k-th approximate) - 2 E_max, with
+//   E_max = (1.01 * 2^-10 + d * 2^-23) |q| dmax  +  1.01 * sqrt(d) * 2^-25 * (dmax / sq + |q| / sd)
+// The first term is the relative rounding of both fp16 images (2^-11 each) plus the fp32 accumulation of d products
+// inside the MMA (d * 2^-23 of sum |q_j d_j|: the worst case of d additions, even if the tensor core truncates; the 1%
+// slack alone would not cover it, 2^-16.6 against up to 2^-12 at d = 4096).  The second is the fp16 underflow floor:
+// the scales sq, sd are one power of two per call / per image, so the elements of a query whose norm is far below the
+// batch's largest become subnormals or zeros, each off by up to 2^-25 / sq absolutely (2^-25 / sd for documents).
+__global__ void flat_margin_kernel(const float* __restrict__ qnorm, int nq, int d, const unsigned* __restrict__ dmax_bits,
+                                   const float* __restrict__ consts, float* __restrict__ margin) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < nq) margin[i] = 2.f * 1.01f * 9.765625e-4f * qnorm[i] * __uint_as_float(*dmax_bits);
+  if (i < nq) {
+    const float dmax = __uint_as_float(*dmax_bits), qn = qnorm[i];
+    const float rel = (1.01f * 9.765625e-4f + (float)d * 1.1920929e-7f) * qn * dmax;
+    const float floor_abs = 1.01f * sqrtf((float)d) * 2.9802322e-8f * (dmax / consts[FC_SQ] + qn / consts[FC_SD]);
+    margin[i] = 2.f * (rel + floor_abs);
+  }
 }
 
 struct GemmParams {
@@ -640,7 +651,7 @@ int mevi_flat_tensor_search_image(mevi_ctx* ctx, const float* Q, int nq, const f
   flat_consts_kernel<<<1, 32, 0, st>>>(docmeta, absmax_q, consts);
   to_fp16_image_kernel<<<ctx->sm_count * 2, 256, 0, st>>>(Q, nq, d, FT_TN, consts, FC_SQ, Bimg, qnorm, nullptr, flags + 2,
                                                           (int64_t)n_qblocks * FT_TN);
-  flat_margin_kernel<<<(nq + 255) / 256, 256, 0, st>>>(qnorm, nq, docmeta + DM_MAXNORM, margin);
+  flat_margin_kernel<<<(nq + 255) / 256, 256, 0, st>>>(qnorm, nq, d, docmeta + DM_MAXNORM, consts, margin);
   MEVI_CUDA(ctx, cudaGetLastError());
   MEVI_COUNT_LAUNCH(ctx, 5);
 
@@ -1127,7 +1138,7 @@ extern "C" int mevi_rerank_grouped_begin(mevi_ctx* ctx, const float* Q, int nq, 
   flat_absmax_kernel<<<ctx->sm_count, 256, 0, st>>>(Q, nq, d, 1, s.absmax + 1);
   gr_consts_kernel<<<1, 32, 0, st>>>(s.absmax, s.consts);
   gr_row_norm_kernel<<<(nq + 7) / 8, 256, 0, st>>>(Q, nq, d, s.qnorm);
-  flat_margin_kernel<<<(nq + 255) / 256, 256, 0, st>>>(s.qnorm, nq, s.absmax + 2, s.margin);
+  flat_margin_kernel<<<(nq + 255) / 256, 256, 0, st>>>(s.qnorm, nq, d, s.absmax + 2, s.consts, s.margin);
   gr_q16_kernel<<<(nq + 7) / 8, 256, 0, st>>>(Q, nq, d, s.consts, s.q16, s.flags + 2);
   MEVI_CUDA(ctx, cudaGetLastError());
   MEVI_COUNT_LAUNCH(ctx, 9);
