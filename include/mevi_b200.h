@@ -77,9 +77,7 @@ int mevi_ctx_check(mevi_ctx* ctx, void* stream);
  *                     (pq.py:304-305 subtracts after every level), or NULL
  *   stats_or_null     int64[8] DEVICE out: [0]=rows re-decided by the exact
  *                     fix-up because their prefilter top-2 gap was inside the
- *                     error bound (tensor mode), [1]=rows processed, [2]=(row, level)
- *                     decisions the hi.hi prefilter left open and the epilogue
- *                     refined with fp32 dot products (generation 6); rest 0   */
+ *                     error bound (tensor mode), [1]=rows processed; rest 0 */
 int mevi_rq_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* codebook, int M, int K,
                    int metric, int mode, int32_t* codes, float* residual_or_null, int64_t* stats_or_null,
                    void* stream);

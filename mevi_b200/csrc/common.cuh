@@ -27,7 +27,6 @@ enum WsSlot {
   WS_MISC,
   WS_PQ_PAD,        // PQ encode on the tensor path: block-padded codebook
   WS_FLAT_IMAGE,    // one-shot flat search: fp16 image of the documents (+ its metadata)
-  WS_RQ_OPEN,       // K1 generation 6: open-row list (rows, state, tensor-core accumulators) for the refine kernel
   WS_GR_PLAN,       // grouped re-rank: device-side round plan (counts, scans, arrival numbers)
   WS_NUM
 };
@@ -51,16 +50,6 @@ struct mevi_ctx {
   // the mirror is inspected at the start of the next call, after every synchronising call, and by mevi_ctx_check.
   int* dev_err = nullptr;            // [MEVI_ERRSLOTS]
   volatile int* host_err = nullptr;  // [MEVI_ERRSLOTS], cudaMallocHost
-  // set by mevi_pq_encode around its call of the RQ tensor kernel on the block-padded codebook: the rows the
-  // prefilter flags are then re-decided by the sub-vector kernel (the PQ reference arithmetic), not by rq_exact
-  const float* pq_fix_codebook = nullptr;
-  int pq_fix_dsub = 0;
-  // set by mevi_kmeans_step_fused around its call of the tensor assignment kernel: the same pass then also accumulates
-  // the rows under their PREVIOUS assignment into per-CTA partial sums | counts ([grid][K][d] floats, [grid][K] ints)
-  const int32_t* km_prev = nullptr;
-  int64_t km_prev_stride = 0;
-  float* km_part_sums = nullptr;
-  int32_t* km_part_counts = nullptr;
   // host-side state of the grouped re-rank's round plan between mevi_rerank_grouped_plan and its _plan_fill calls
   // (rerank_plan.cu owns the layout; malloc'ed, freed with the context)
   void* gr_plan = nullptr;
@@ -77,6 +66,46 @@ int mevi_deferred_error(mevi_ctx* ctx);
 // grow-on-demand scratch; returns nullptr (and sets the error) on failure
 void* mevi_ws(mevi_ctx* ctx, int slot, size_t bytes);
 void* mevi_pinned(mevi_ctx* ctx, int slot, size_t bytes);
+
+// ---- internal entry points called across kernel files (the C ABI is include/mevi_b200.h) ----------------------
+// rq_exact.cu: fp32 direct-form RQ encode / k-means assignment, of all rows or of the rows of a device-side work list
+int mevi_rq_exact_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
+                         int32_t* codes, int64_t codes_stride, float* residual, const int32_t* work_rows,
+                         const int32_t* work_levels, const int64_t* n_work_dev, int64_t n_items, double* inertia,
+                         cudaStream_t st);
+
+// rq_tensor.cu: K1 (tcgen05 RQ encode / k-means assignment) and the wide-codebook PQ encode
+// The fused k-means pass: the assignment pass also accumulates the rows under their PREVIOUS assignment into per-CTA
+// partial sums | counts ([grid][K][d] floats, [grid][K] ints; grid = min(ceil(n / 256), SM count)).
+struct KmeansFusedPass {
+  const int32_t* prev;
+  int64_t prev_stride;
+  float* part_sums;
+  int32_t* part_counts;
+};
+bool mevi_rq_tensor_supported(mevi_ctx* ctx, int d, int M, int K, int metric);
+bool mevi_kmeans_fused_supported(mevi_ctx* ctx, int d, int K);
+// pq_codebook: when non-null, codes are PQ codes of a block-padded `cb` and the rows the prefilter flags are re-decided
+// by the sub-vector kernel against this [M][K][d/M] codebook instead of by rq_exact.  km_fused: non-null (M = 1 only)
+// runs the fused k-means pass.
+int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
+                          int32_t* codes, int64_t codes_stride, float* residual, int64_t* stats, double* inertia,
+                          const float* pq_codebook, const KmeansFusedPass* km_fused, cudaStream_t st);
+bool mevi_pq_tensor_supported(mevi_ctx* ctx, int64_t n, int d, int M, int K, int metric);
+int mevi_pq_tensor_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
+                          int32_t* codes, cudaStream_t st);
+
+// pq_encode.cu: the fp32 sub-vector kernel as the arbiter of the tensor PQ routes
+int mevi_pq_fix_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* pq_codebook, int M, int K, int metric,
+                       int32_t* codes, const int32_t* work_rows, const int64_t* n_work_dev, cudaStream_t st);
+int mevi_pq_fix_pairs_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* pq_codebook, int M, int K, int metric,
+                             int32_t* codes, const uint32_t* pairs, const unsigned long long* n_pairs_dev, unsigned long long cap,
+                             const int* overflow, cudaStream_t st);
+
+// flat_tensor.cu: K2 on the tensor cores (*fell_back = 1: the fp32 path has to compute the answer)
+bool mevi_flat_tensor_supported(mevi_ctx* ctx, int d, int k);
+int mevi_flat_tensor_search(mevi_ctx* ctx, const float* Q, int nq, const float* D, int64_t n, int d, int k,
+                            int64_t id_base, float* scores, int64_t* ids, int* fell_back, cudaStream_t st);
 
 #define MEVI_COUNT_LAUNCH(ctx, n) ((ctx)->launches += (n))
 

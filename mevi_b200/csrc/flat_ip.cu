@@ -18,9 +18,6 @@
 
 #include "common.cuh"
 
-int mevi_topk_merge_launch(mevi_ctx* ctx, const float* in_s, const int64_t* in_i, int S, int nq, int k,
-                           int64_t list_stride, int64_t shard_stride, float* out_s, int64_t* out_i, cudaStream_t st);
-
 namespace {
 
 constexpr int FT_BM = 128, FT_BN = 128, FT_BK = 16, FT_THREADS = 256;
@@ -163,10 +160,6 @@ int pow2_at_least(int v) {
 }
 
 }  // namespace
-
-bool mevi_flat_tensor_supported(mevi_ctx* ctx, int d, int k);
-int mevi_flat_tensor_search(mevi_ctx* ctx, const float* Q, int nq, const float* D, int64_t n, int d, int k,
-                            int64_t id_base, float* scores, int64_t* ids, int* fell_back, cudaStream_t st);
 
 extern "C" int mevi_flat_ip_topk(mevi_ctx* ctx, const float* Q, int nq, const float* D, int64_t n, int d, int k,
                                  int64_t id_base, int mode, float* scores, int64_t* ids, void* stream) {

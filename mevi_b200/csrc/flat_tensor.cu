@@ -20,7 +20,6 @@
 // blocks.  Roofline: tensor pipe (2*nq*N*d FLOP); L2->SM operand traffic is the practical limiter.
 #include <cuda_fp16.h>
 #include <math_constants.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -660,9 +659,8 @@ int mevi_flat_tensor_search_image(mevi_ctx* ctx, const float* Q, int nq, const f
   p.consts = consts; p.tau = tau; p.margin = margin; p.count = count; p.cand_score = cand_score; p.cand_id = cand_id;
   p.overflow = flags; p.capg = capg; p.err_flag = flags + 1;
   const size_t smem_gemm = (size_t)FT_STAGES * FT_STAGE_BYTES + 2 * FT_TN * 4 + (2 * FT_STAGES + 4) * 8 + 16 + 1024;
-  // cluster size: MEVI_FLAT_CLUSTER=1|2|4 overrides the default
+  // cluster size: FT_DEFAULT_CLUSTER, or 1 when no cluster of that size can be resident
   int cs = FT_DEFAULT_CLUSTER;
-  if (const char* e = getenv("MEVI_FLAT_CLUSTER")) cs = atoi(e);
   int max_clusters = cs == 4 ? flat_max_clusters<4>(ctx, smem_gemm) : cs == 2 ? flat_max_clusters<2>(ctx, smem_gemm) : 0;
   if (max_clusters <= 0) { cs = 1; max_clusters = ctx->sm_count; }
   const size_t smem_compact = (size_t)capg * 8;

@@ -15,22 +15,11 @@
 // are then reduced in a fixed order.  No float atomics, so sums are
 // bit-reproducible for a given (n, grid) and ranks stay in lockstep.
 // Roofline: HBM (one more read of the shard: 4*d bytes per row + 4 B assignment).
-#include <stdlib.h>
 
 #include <cub/cub.cuh>
 
 #include "common.cuh"
 #include "ptx.cuh"
-
-int mevi_rq_exact_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                         int32_t* codes, int64_t codes_stride, float* residual, const int32_t* work_rows,
-                         const int32_t* work_levels, const int64_t* n_work_dev, int64_t n_items, double* inertia,
-                         cudaStream_t st);
-int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                          int32_t* codes, int64_t codes_stride, float* residual, int64_t* stats, double* inertia,
-                          cudaStream_t st);
-bool mevi_rq_tensor_supported(mevi_ctx* ctx, int d, int M, int K, int metric);
-bool mevi_kmeans_fused_supported(mevi_ctx* ctx, int d, int K);
 
 namespace {
 
@@ -39,6 +28,7 @@ constexpr int KM_WARPS = KM_THREADS / 32;
 constexpr int KM_TILE = 256;
 constexpr int KA_MAX_STAGES = 8;
 constexpr int KA_DEFAULT_STAGES = 2;  // shared-memory stages of the accumulate kernel (stages-1 bulk copies in flight)
+static_assert(KA_DEFAULT_STAGES >= 2 && KA_DEFAULT_STAGES <= KA_MAX_STAGES, "the accumulate kernel's barrier arrays hold KA_MAX_STAGES");
 
 // Column-owner accumulation (skew-proof and deterministic).  The CTA keeps the running [K][d] fp32
 // sums in shared memory; thread t owns column t of every centroid.  Rows arrive in sub-tiles — one
@@ -214,10 +204,7 @@ int accumulate_by_code(mevi_ctx* ctx, const float* R, int64_t n, int d, const in
   const int64_t kd = (int64_t)K * d;
   // shared-memory budget: [K][d] accumulators + KA_STAGES stages of sub_rows rows
   const size_t acc_bytes = (size_t)kd * sizeof(float);
-  int KA_STAGES = KA_DEFAULT_STAGES;
-  if (const char* e = getenv("MEVI_KA_STAGES")) KA_STAGES = atoi(e);
-  if (KA_STAGES < 2) KA_STAGES = 2;
-  if (KA_STAGES > KA_MAX_STAGES) KA_STAGES = KA_MAX_STAGES;
+  const int KA_STAGES = KA_DEFAULT_STAGES;
   int sub_rows = acc_bytes + 4096 < 220 * 1024 ? (int)((220 * 1024 - acc_bytes) / ((size_t)KA_STAGES * d * 4)) : 0;
   if (sub_rows > 32) sub_rows = 32;
   const bool fast = K <= 64 && d <= 992 && d % 4 == 0 && sub_rows >= 4 && (reinterpret_cast<uintptr_t>(R) & 15) == 0;
@@ -394,7 +381,7 @@ int mevi_kmeans_step(mevi_ctx* ctx, const float* R, int64_t n, int d, const floa
   int rc;
   if (use_tensor)
     rc = mevi_rq_tensor_assign(ctx, R, n, d, centroids, 1, K, MEVI_METRIC_L2, assign, stride, nullptr, nullptr,
-                               inertia_or_null, st);
+                               inertia_or_null, nullptr, nullptr, st);
   else
     rc = mevi_rq_exact_launch(ctx, R, n, d, centroids, 1, K, MEVI_METRIC_L2, assign, stride, nullptr, nullptr, nullptr,
                               nullptr, n, inertia_or_null, st);
@@ -425,13 +412,9 @@ int mevi_kmeans_step_fused(mevi_ctx* ctx, const float* R, int64_t n, int d, cons
   const size_t ps_bytes = (size_t)G * kd * sizeof(float), pc_bytes = (size_t)G * K * sizeof(int32_t);
   char* ws = (char*)mevi_ws(ctx, WS_KM_PARTIAL, ps_bytes + pc_bytes);
   if (!ws) return MEVI_ERR_NOMEM;
-  ctx->km_prev = prev_assign;
-  ctx->km_prev_stride = prev_stride;
-  ctx->km_part_sums = (float*)ws;
-  ctx->km_part_counts = (int32_t*)(ws + ps_bytes);
+  const KmeansFusedPass fused = {prev_assign, prev_stride, (float*)ws, (int32_t*)(ws + ps_bytes)};
   const int rc = mevi_rq_tensor_assign(ctx, R, n, d, centroids, 1, K, MEVI_METRIC_L2, assign_out, assign_stride, nullptr, nullptr,
-                                       inertia_or_null, st);
-  ctx->km_prev = nullptr;
+                                       inertia_or_null, nullptr, &fused, st);
   if (rc != MEVI_OK) return rc;
   const int threads = 256;
   kmeans_reduce_partials_kernel<<<(int)((kd + K + threads - 1) / threads), threads, 0, st>>>((const float*)ws, (const int32_t*)(ws + ps_bytes),
@@ -471,7 +454,7 @@ int mevi_kmeans_step_delta(mevi_ctx* ctx, const float* R, int64_t n, int d, cons
   int rc;
   if (use_tensor)
     rc = mevi_rq_tensor_assign(ctx, R, n, d, centroids, 1, K, MEVI_METRIC_L2, assign_out, assign_stride, nullptr, nullptr,
-                               inertia_or_null, st);
+                               inertia_or_null, nullptr, nullptr, st);
   else
     rc = mevi_rq_exact_launch(ctx, R, n, d, centroids, 1, K, MEVI_METRIC_L2, assign_out, assign_stride, nullptr, nullptr, nullptr,
                               nullptr, n, inertia_or_null, st);

@@ -230,14 +230,6 @@ __global__ void pq_pad_codebook_kernel(const float* __restrict__ cb, int M, int 
 }
 }  // namespace
 
-int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                          int32_t* codes, int64_t codes_stride, float* residual, int64_t* stats, double* inertia,
-                          cudaStream_t st);
-bool mevi_rq_tensor_supported(mevi_ctx* ctx, int d, int M, int K, int metric);
-bool mevi_pq_tensor_supported(mevi_ctx* ctx, int64_t n, int d, int M, int K, int metric);
-int mevi_pq_tensor_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* codebook, int M, int K, int metric,
-                          int32_t* codes, int64_t* stats, cudaStream_t st);
-
 extern "C" int mevi_pq_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* codebook, int M, int K,
                               int metric, int32_t* codes, void* stream) {
   MEVI_CHECK_CTX(ctx);
@@ -261,15 +253,10 @@ extern "C" int mevi_pq_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, c
     pq_pad_codebook_kernel<<<ctx->sm_count, 256, 0, st>>>(codebook, M, K, dsub, padded);
     MEVI_CUDA(ctx, cudaGetLastError());
     MEVI_COUNT_LAUNCH(ctx, 1);
-    ctx->pq_fix_codebook = codebook;
-    ctx->pq_fix_dsub = dsub;
-    const int rc = mevi_rq_tensor_assign(ctx, X, n, d, padded, M, K, metric, codes, M, nullptr, nullptr, nullptr, st);
-    ctx->pq_fix_codebook = nullptr;
-    ctx->pq_fix_dsub = 0;
-    return rc;
+    return mevi_rq_tensor_assign(ctx, X, n, d, padded, M, K, metric, codes, M, nullptr, nullptr, nullptr, codebook, nullptr, st);
   }
   // wide codebooks (K = 256, sub-vector width 32): the split-fp16 tensor kernel of pq_tensor.cuh
   if (!(env && atoi(env) == 0) && n >= 4096 && mevi_pq_tensor_supported(ctx, n, d, M, K, metric))
-    return mevi_pq_tensor_encode(ctx, X, n, d, codebook, M, K, metric, codes, nullptr, st);
+    return mevi_pq_tensor_encode(ctx, X, n, d, codebook, M, K, metric, codes, st);
   return launch_pq_kernel(ctx, X, n, d, codebook, M, K, metric, codes, nullptr, nullptr, st);
 }

@@ -58,18 +58,7 @@ struct PqParams {
   uint32_t* pairs; unsigned long long* pair_count; unsigned long long pair_cap; int* overflow;
   int* err_flag;
   int64_t n_tiles;
-  int debug;
-  unsigned long long* trace;  // MEVI_PQ_TRACE=<file>: per-warp event clocks of CTA 0 for sub-vector steps [TRQ0, TRQ1)
 };
-
-// pipeline trace (debug aid): lane 0 of every warp of CTA 0 appends (clock << 16 | event << 12 | step) for a window of steps
-constexpr int TRQ_SLOTS = 128, TRQ_WARPS = 16, TRQ0 = 40, TRQ1 = 52;
-__device__ __forceinline__ void trq(const PqParams& p, int warp, int lane, uint32_t& idx, uint32_t q, uint32_t ev) {
-  if (p.trace != nullptr && blockIdx.x == 0 && lane == 0 && q >= TRQ0 && q < TRQ1 && idx < TRQ_SLOTS) {
-    p.trace[warp * TRQ_SLOTS + idx] = ((unsigned long long)clock64() << 16) | (ev << 12) | (q & 4095u);
-    ++idx;
-  }
-}
 
 struct SmemQ {
   int x_off, b_off, subc_off, norm_off, bar_off, holder_off, total;
@@ -153,23 +142,18 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
 
   if (warp == 0) {
     // ===== TMA producer: one [128 x 32] fp32 box per (group, tile, sub-vector) =====
-    uint32_t s = 0, ph = 0, tq = 0, tix = 0;
+    uint32_t s = 0, ph = 0;
     for (int g = 0; g < ngroups; ++g) {
       const int gs = M - g * GSQ < GSQ ? M - g * GSQ : GSQ;
       for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
-        for (int sv = 0; sv < gs; ++sv, ++tq) {
+        for (int sv = 0; sv < gs; ++sv) {
           if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait_backoff(&x_empty[s], ph ^ 1, 32))) {
             if (lane == 0) atomicExch(p.err_flag, 1);
             return;
           }
-          trq(p, warp, lane, tix, tq, 0);
           if (ptx::elect_one()) {
-            if (p.debug & 16) {  // experiment: no HBM traffic (the stage keeps whatever it holds)
-              ptx::mbar_arrive(&x_full[s]);
-            } else {
-              ptx::mbar_arrive_expect_tx(&x_full[s], TMQ * DS * 4);
-              ptx::tma_load_2d(sX + (size_t)s * X_STAGEQ, &tmap, (g * GSQ + sv) * DS, (int)(tile * TMQ), &x_full[s]);
-            }
+            ptx::mbar_arrive_expect_tx(&x_full[s], TMQ * DS * 4);
+            ptx::tma_load_2d(sX + (size_t)s * X_STAGEQ, &tmap, (g * GSQ + sv) * DS, (int)(tile * TMQ), &x_full[s]);
           }
           __syncwarp();
           if (++s == NSXQ) { s = 0; ph ^= 1; }
@@ -196,7 +180,7 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
     // ===== MMA: warp h issues the units (sub-vector, half h); unit u = 2q + h lives in accumulator buffer u % 3 =====
     const int h = warp - 1;
     const uint32_t idesc = ptx::umma_idesc_f16_m128(128u);
-    uint32_t as = 0, aph = 0, q = 0, buf = (uint32_t)h, ebits = 0, tix = 0;
+    uint32_t as = 0, aph = 0, q = 0, buf = (uint32_t)h, ebits = 0;
     for (int g = 0; g < ngroups; ++g) {
       const int gs = M - g * GSQ < GSQ ? M - g * GSQ : GSQ;
       if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait_backoff(b_full, g & 1, 32))) {
@@ -215,33 +199,28 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
             ebits ^= 1u << buf;
           }
           const uint32_t d_tmem = tmem_base + buf * 128u;
-          trq(p, warp, lane, tix, q, 0);
           if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait(&a_full[as], aph))) {
             if (lane == 0) atomicExch(p.err_flag, 3);
             return;
           }
-          trq(p, warp, lane, tix, q, 1);
           ptx::tc_fence_after_sync();
           const uint32_t b_hi = ptx::smem_u32(sB + (size_t)sv * B_SUBQ) + (uint32_t)h * 128u * 64u;
           const uint32_t b_lo = b_hi + (uint32_t)B_BLOCKQ, b_bias = b_lo + (uint32_t)B_BLOCKQ;
           if (ptx::elect_one()) {
-            if (!(p.debug & 2)) {
-              const uint32_t a_hi = tmem_base + AQ_COL0 + as * 32, a_lo = a_hi + 16;
-              // scores = -|c_k|^2 (constant tile x bias block) + 2 x.c (the scales carry the factor): 7 MMAs
-              ptx::umma_f16_ts(d_tmem, tmem_base + AQ_CONST, ptx::umma_desc_sw64(b_bias), idesc, 0u);
+            const uint32_t a_hi = tmem_base + AQ_COL0 + as * 32, a_lo = a_hi + 16;
+            // scores = -|c_k|^2 (constant tile x bias block) + 2 x.c (the scales carry the factor): 7 MMAs
+            ptx::umma_f16_ts(d_tmem, tmem_base + AQ_CONST, ptx::umma_desc_sw64(b_bias), idesc, 0u);
 #pragma unroll
-              for (int ks = 0; ks < DSQ / 16; ++ks) {
-                ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, 1u);
-                ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_lo + ks * 32), idesc, 1u);
-                ptx::umma_f16_ts(d_tmem, a_lo + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, 1u);
-              }
+            for (int ks = 0; ks < DSQ / 16; ++ks) {
+              ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, 1u);
+              ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_lo + ks * 32), idesc, 1u);
+              ptx::umma_f16_ts(d_tmem, a_lo + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, 1u);
             }
             ptx::umma_commit(&a_empty[as]);
             ptx::umma_commit(&acc_full[2 * buf + (q & 1)]);
             if (last_tile && sv == gs - 1) ptx::umma_commit(b_free);
           }
           __syncwarp();
-          trq(p, warp, lane, tix, q, 2);
           if (++as == NSAQ) { as = 0; aph ^= 1; }
           buf = buf >= 1 ? buf - 1 : buf + 2;  // (u + 2) % 3
         }
@@ -265,15 +244,13 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
       for (int i = 2; i < 16; ++i) ct[i] = 0u;
       ptx::tmem_st16(t_lane + AQ_CONST, ct);  // columns 480-495 (only 480-487 are read)
     }
-    uint32_t xs = 0, xph = 0, as = 0, aph = 0, q = 0, tix = 0;
+    uint32_t xs = 0, xph = 0, as = 0, aph = 0, q = 0;
     for (int g = 0; g < ngroups; ++g) {
       const int gs = M - g * GSQ < GSQ ? M - g * GSQ : GSQ;
       for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
         for (int sv = 0; sv < gs; ++sv, ++q) {
           if (!ptx::mbar_wait(&x_full[xs], xph)) { atomicExch(p.err_flag, 4); return; }
-          trq(p, warp, lane, tix, q, 0);
           if (!ptx::mbar_wait_backoff(&a_empty[as], aph ^ 1, 32)) { atomicExch(p.err_flag, 4); return; }
-          trq(p, warp, lane, tix, q, 1);
           ptx::tc_fence_after_sync();
           uint32_t hi[16], lo[16];
           float2 norm2 = make_float2(0.f, 0.f);
@@ -283,9 +260,6 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
             if (4 * j >= DS) {  // K padding of the narrow sub-vector
               hi[2 * j] = hi[2 * j + 1] = lo[2 * j] = lo[2 * j + 1] = 0u;
               continue;
-            }
-            if (p.debug & 8) {  // experiment: no conversion work (one load, constant operands)
-              if (j > 0) { hi[2 * j] = hi[0]; hi[2 * j + 1] = hi[1]; lo[2 * j] = lo[0]; lo[2 * j + 1] = lo[1]; continue; }
             }
             asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(p01.x), "=f"(p01.y), "=f"(p23.x), "=f"(p23.y)
                          : "r"(src_row + xs * X_STAGEQ + (((uint32_t)j ^ sw) << 4)));
@@ -312,7 +286,6 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
           ptx::tc_fence_before_sync();
           __syncwarp();
           if (lane == 0) { ptx::mbar_arrive(&a_full[as]); ptx::mbar_arrive(&st_full[q & (NORMQ - 1)]); }
-          trq(p, warp, lane, tix, q, 2);
           if (++xs == NSXQ) { xs = 0; xph ^= 1; }
           if (++as == NSAQ) { as = 0; aph ^= 1; }
         }
@@ -328,14 +301,16 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
     // |x_j|^2 below this guarantees that no scaled element overflowed the fp16 range
     const float xn2_limit = 65000.f * 65000.f * p.consts[C_INV_SX2];
     const uint32_t taddr = tmem_base + ((uint32_t)(qd * 32) << 16);
-    const bool math = !(p.debug & 4);
-    uint32_t q = 0, fbits = 0, tix = 0;
+    uint32_t q = 0, fbits = 0;
     bool ok = true;
     for (int g = 0; g < ngroups && ok; ++g) {
       const int gs = M - g * GSQ < GSQ ? M - g * GSQ : GSQ;
       if (!ptx::mbar_wait_backoff(b_full, g & 1, 64)) { atomicExch(p.err_flag, 6); ok = false; break; }
       for (int64_t tile = blockIdx.x; tile < p.n_tiles && ok; tile += gridDim.x) {
         const int64_t row = tile * TMQ + rl;
+        // a warp whose rows all lie past the end has nothing to reduce.  The branch also keeps ptxas from hoisting the
+        // second tcgen05.ld above the first reduction: two live 64-score sets do not fit 128 registers and spill.
+        const bool live = __any_sync(MEVI_FULL_MASK, row < p.n);
         for (int sv = 0; sv < gs; ++sv, ++q) {
           if ((int)(q & 1) != e) continue;
           // scores as a 16 x 16 matrix (k = 16 g + j): row maxima R[g], column maxima C[j]
@@ -347,20 +322,18 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
             const uint32_t buf = (2 * q + h) % NACCQ;
             if (!ptx::mbar_wait_backoff(&acc_full[2 * buf + e], (fbits >> buf) & 1u, 20)) { atomicExch(p.err_flag, 6); ok = false; break; }
             fbits ^= 1u << buf;
-            trq(p, warp, lane, tix, q, 2 * h);
             ptx::tc_fence_after_sync();
             uint32_t ra[64];
             ptx::tmem_ld64(taddr + buf * 128u, ra);
             ptx::tmem_ld_wait();
-            if (math) reduce64(ra, 2 * h, R, C);
+            if (live) reduce64(ra, 2 * h, R, C);
             ptx::tmem_ld64(taddr + buf * 128u + 64u, ra);
             ptx::tmem_ld_wait();
             // the unit is in registers: hand the buffer to its next tenant (unit u + 3, the other half's MMA warp)
             ptx::tc_fence_before_sync();
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(&acc_empty[2 * buf + (h ^ 1)]);
-            trq(p, warp, lane, tix, q, 2 * h + 1);
-            if (math) reduce64(ra, 2 * h + 1, R, C);
+            if (live) reduce64(ra, 2 * h + 1, R, C);
           }
           if (!ok) break;
           if (!ptx::mbar_wait_backoff(&st_full[q & (NORMQ - 1)], (q >> 4) & 1, 32)) { atomicExch(p.err_flag, 6); ok = false; break; }
@@ -388,7 +361,7 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
           const bool valid = row < p.n;
           const int m = g * GSQ + sv;
           if (valid) p.codes[row * M + m] = gi * 16 + ji;
-          const bool flag = valid && !decided && math;
+          const bool flag = valid && !decided;
           const unsigned fm = __ballot_sync(MEVI_FULL_MASK, flag);
           if (fm != 0u) {
             const int leader = __ffs(fm) - 1;
@@ -401,7 +374,6 @@ __global__ void __launch_bounds__(THREADSQ, 1) pq_tensor_kernel(PqParams p, cons
               else atomicExch(p.overflow, 1);
             }
           }
-          trq(p, warp, lane, tix, q, 4);
         }
       }
       // the group's images and constants may be overwritten once every epilogue warp (and both MMA warps) are done

@@ -537,7 +537,7 @@ cudaError_t launch_rerank(const RerankParams& p, size_t smem, cudaStream_t st) {
 
 }  // namespace
 
-// internal: merge with explicit strides (used by re-rank splits, flat search and the public merge)
+// internal: merge with explicit strides (used by re-rank splits and the public merge)
 int mevi_topk_merge_launch(mevi_ctx* ctx, const float* in_s, const int64_t* in_i, int S, int nq, int k,
                            int64_t list_stride, int64_t shard_stride, float* out_s, int64_t* out_i, cudaStream_t st) {
   const int cap = next_pow2(S * k);

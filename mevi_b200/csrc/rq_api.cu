@@ -1,15 +1,6 @@
 // rq_api.cu — C-ABI entry points of the RQ encode (device- and host-buffer forms).
 #include "common.cuh"
 
-int mevi_rq_exact_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                         int32_t* codes, int64_t codes_stride, float* residual, const int32_t* work_rows,
-                         const int32_t* work_levels, const int64_t* n_work_dev, int64_t n_items, double* inertia,
-                         cudaStream_t st);
-int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                          int32_t* codes, int64_t codes_stride, float* residual, int64_t* stats, double* inertia,
-                          cudaStream_t st);
-bool mevi_rq_tensor_supported(mevi_ctx* ctx, int d, int M, int K, int metric);
-
 namespace {
 __global__ void stats_add_kernel(int64_t* stats, int64_t flagged, int64_t rows) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
@@ -32,7 +23,8 @@ int encode_dispatch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float
   } else if (mode != MEVI_MODE_EXACT) {
     return mevi_set_error(ctx, MEVI_ERR_INVALID, "unknown mode %d", mode);
   }
-  if (use_tensor) return mevi_rq_tensor_assign(ctx, X, n, d, cb, M, K, metric, codes, M, residual, stats_accum, nullptr, st);
+  if (use_tensor)
+    return mevi_rq_tensor_assign(ctx, X, n, d, cb, M, K, metric, codes, M, residual, stats_accum, nullptr, nullptr, nullptr, st);
   int rc = mevi_rq_exact_launch(ctx, X, n, d, cb, M, K, metric, codes, M, residual, nullptr, nullptr, nullptr, n, nullptr, st);
   if (rc != MEVI_OK) return rc;
   if (stats_accum) {

@@ -13,36 +13,17 @@
 // re-decided with more precision, and rows that stay inside the tightest bound go to a work list for the fp32
 // direct-form kernel of rq_exact.cu, the literal restatement of the reference arithmetic.  Rows outside the bounds
 // provably have the same argmin in exact arithmetic, so codes agree with the reference except at fp32-epsilon ties.
-// Two kernels share this protocol (DESIGN.md section 4 has the measurements that led here):
-//   * generation 4 (rq_tensor4.cuh; the default for every supported shape): split-fp16 contraction hi.hi + hi.lo + lo.hi
-//     (22 significant bits, ~2^-22 |x||c| error) with the document operand in tensor memory; runs the M = 1 k-means
-//     assignment at the HBM roofline and the M = 4 encode at 0.62-0.69 of it (tensor work under the power cap).
-//   * generation 6 (experiments/rq_tensor6.cuh; NOT part of the shipped library: build with `make GEN6=1`, then M >= 2,
-//     K == 32 and MEVI_RQ_KERNEL=6 select it): ONE fp16 MMA per K step (hi.hi) with a
-//     per-row bound built from the measured norm of the row's fp16 remainder; rows with a level the bound leaves open
-//     (11.9 % on N(0,1) data) are dumped with their tensor-core accumulators and finished by rq_refine6_kernel (exact fp32
-//     dot products of the open candidates), or refined inside the epilogue (MEVI_RQ_REFINE=inline).  Bit-identical codes,
-//     a third of the tensor work, but not faster end to end (7.3 ms vs 6.5 ms): kept as a measured alternative.
+// The kernel (rq_tensor4.cuh, generation 4) contracts in split fp16, hi.hi + hi.lo + lo.hi (22 significant bits,
+// ~2^-22 |x||c| error), with the document operand in tensor memory; it runs the M = 1 k-means assignment at the HBM
+// roofline and the M = 4 encode at 0.62-0.69 of it (tensor work under the power cap).  DESIGN.md section 4 has the
+// measurements that led here, including those of the slower alternatives.
 // Roofline: HBM (4*d B/row).
 #include <cuda.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <cstdio>
-#include <vector>
 #include <math_constants.h>
 
 #include "common.cuh"
 #include "ptx.cuh"
-
-int mevi_rq_exact_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                         int32_t* codes, int64_t codes_stride, float* residual, const int32_t* work_rows,
-                         const int32_t* work_levels, const int64_t* n_work_dev, int64_t n_items, double* inertia,
-                         cudaStream_t st);
-int mevi_pq_fix_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* pq_codebook, int M, int K, int metric,
-                       int32_t* codes, const int32_t* work_rows, const int64_t* n_work_dev, cudaStream_t st);
-int mevi_pq_fix_pairs_launch(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* pq_codebook, int M, int K, int metric,
-                             int32_t* codes, const uint32_t* pairs, const unsigned long long* n_pairs_dev, unsigned long long cap,
-                             const int* overflow, cudaStream_t st);
 
 namespace {
 
@@ -55,47 +36,15 @@ enum { C_SC = 0, C_SX, C_INV, C_INV_SX2, C_FX, C_FC, C_NUM = 8 };
 struct Params {
   const float* X; int64_t n; int d; int nchunks;
   int M, K, NT, N1, metric;
-  const float* cb;  // fp32 codebook [M*K][d] (generation 6 refines against it)
   const __half* Bimg; const float* cn2; const float* e1; const float* lvl; const float* gram; const float* consts;
-  const float* ea1; const float* ea2;  // generation 6: per-candidate constants of the hi.hi bound
   int gram_floats;
   int32_t* codes; int64_t codes_stride;
   int32_t* work_rows; int32_t* work_levels; unsigned long long* work_count;
-  unsigned long long* refine_count;  // generation 6: (row, level) decisions refined in the epilogue
-  // generation 6, two-kernel form: rows with an open level are dumped (row, state, tensor-core accumulators of all levels)
-  // for rq_refine6_kernel instead of being refined inside the epilogue
-  int32_t* open_rows; int4* open_meta; float* open_t1; unsigned long long* open_count; int64_t open_cap;
   // fused k-means pass (rq_tensor4_kernel<1, true>): previous assignment in, per-CTA partial sums | counts out
   const int32_t* prev; int64_t prev_stride; float* part_sums; int32_t* part_counts;
   double* inertia; int* err_flag;
   int64_t n_tiles;
-  int debug;  // MEVI_RQ_DEBUG bit mask for pipeline ablations (timing experiments only; results are wrong)
-  unsigned long long* trace;  // MEVI_RQ_TRACE=<file>: per-warp event timestamps of CTA 0 (pipeline debugging), else null
 };
-
-// Pipeline trace (debug aid): lane 0 of every warp of CTA 0 appends (clock << 16 | event << 12 | tile_it << 8 | chunk)
-// for tile iterations [TRACE_IT0, TRACE_IT1).  tools/rq_trace.py turns the dump into a per-role timeline.
-constexpr int TRACE_SLOTS = 512, TRACE_WARPS = 20, TRACE_IT0 = 6, TRACE_IT1 = 9;
-// (SM clock, global nanosecond timer) at the start (which = 0) and end (which = 1) of CTA 0: the SM clock the kernel really ran at
-__device__ __forceinline__ void trace_clock(const Params& p, int which) {
-  if (p.trace != nullptr && blockIdx.x == 0 && threadIdx.x == 0) {
-    unsigned long long ns;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    p.trace[TRACE_SLOTS * TRACE_WARPS + 2 * which] = (unsigned long long)clock64();
-    p.trace[TRACE_SLOTS * TRACE_WARPS + 2 * which + 1] = ns;
-  }
-}
-__device__ __forceinline__ void trace_ev(const Params& p, int warp, int lane, uint32_t& idx, uint32_t it, uint32_t c, uint32_t ev) {
-  if (p.trace != nullptr && blockIdx.x == 0 && lane == 0 && it >= TRACE_IT0 && it < TRACE_IT1 && idx < TRACE_SLOTS) {
-    p.trace[warp * TRACE_SLOTS + idx] = ((unsigned long long)clock64() << 16) | (ev << 12) | ((it & 15u) << 8) | (c & 255u);
-    ++idx;
-  }
-}
-
-template <int N>
-__device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
-template <int N>
-__device__ __forceinline__ void reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
 
 // ---- preparation kernels ---------------------------------------------------------------------
 __global__ void absmax_kernel(const float* __restrict__ p, int64_t rows, int d, int64_t row_step, unsigned* out) {
@@ -205,12 +154,10 @@ __global__ void level_consts_kernel(const float* __restrict__ cnorm, const float
   }
 }
 
-__global__ void finish_stats_kernel(const unsigned long long* work_count, const unsigned long long* refine_count, int64_t rows,
-                                    int64_t* stats) {
+__global__ void finish_stats_kernel(const unsigned long long* work_count, int64_t rows, int64_t* stats) {
   if (threadIdx.x == 0 && blockIdx.x == 0 && stats) {
     atomicAdd((unsigned long long*)&stats[0], *work_count);
     atomicAdd((unsigned long long*)&stats[1], (unsigned long long)rows);
-    atomicAdd((unsigned long long*)&stats[2], *refine_count);
   }
 }
 
@@ -257,41 +204,6 @@ __global__ void bimg32_kernel(const float* __restrict__ cb, int rows_valid, int 
   }
 }
 
-// one warp per centroid row: cl[r] = | c*sc - fp16(c*sc) | / sc, the norm of what the fp16 image of the centroid drops
-// (exact: the subtraction is exact in fp32, the sum is taken in double).  Input of the hi.hi prefilter's error bound.
-__global__ void clo_norm_kernel(const float* __restrict__ cb, int rows_valid, int d, int NT, const float* __restrict__ consts,
-                                float* __restrict__ cl) {
-  const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (r >= NT) return;
-  const float sc = consts[C_SC];
-  double s = 0.0;
-  if (r < rows_valid)
-    for (int c = threadIdx.x & 31; c < d; c += 32) {
-      const float t = cb[(size_t)r * d + c] * sc;
-      const double lo = (double)(t - __half2float(__float2half_rn(t)));
-      s += lo * lo;
-    }
-  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(MEVI_FULL_MASK, s, o);
-  if ((threadIdx.x & 31) == 0) cl[r] = (float)(sqrt(s) / (double)sc * (1.0 + 1e-6));
-}
-
-// Error model of the hi.hi prefilter (generation 6).  With x*sx = xh + xl (xh = fp16(x*sx), xl the exact fp32 remainder)
-// and c*sc = ch + cl likewise, the tensor cores contract xh.ch with exact products and fp32 accumulation, so
-//   | xh.ch/(sx sc) - x.c |  <=  a |c| + (|x| + a) cl_k + U_REL |x| |c|,      a = |xl|/sx  (measured per row)
-// In distance units (f = 2 for L2, 1 for IP) the per-candidate bound is  a * EA1_k + |x| * EA2_k  (+ B_j/2 for the fp32
-// epilogue, the same level constant as the tight bound):
-//   EA1_k = f (|c_k| + cl_k) (1 + 2^-12)          (the slack covers the fp32 rounding of the measured a and |x|)
-//   EA2_k = f (cl_k + (U_REL + EPS_A) |c_k|) (1 + 2^-12)
-__global__ void loose_consts_kernel(const float* __restrict__ cnorm, const float* __restrict__ cl, int NT, int metric,
-                                    float* __restrict__ ea1, float* __restrict__ ea2) {
-  const int k = blockIdx.x * blockDim.x + threadIdx.x;
-  if (k >= NT) return;
-  const float f = metric == MEVI_METRIC_L2 ? 2.f : 1.f;
-  const float slack = 1.f + 1.f / 4096.f;
-  ea1[k] = f * (cnorm[k] + cl[k]) * slack;
-  ea2[k] = f * (cl[k] + (U_REL + 4.8e-7f) * cnorm[k]) * slack;
-}
-
 // after the encode kernel: a pipeline time-out (err != 0) must never leave plausible-looking codes behind
 __global__ void poison_codes_kernel(const int* __restrict__ err, int32_t* __restrict__ codes, int64_t n, int64_t stride, int M) {
   if (*err == 0) return;
@@ -329,9 +241,6 @@ inline int make_x_tensormap(mevi_ctx* ctx, const float* X, int64_t n, int d, int
 }
 
 #include "rq_tensor4.cuh"
-#ifdef MEVI_WITH_GEN6
-#include "experiments/rq_tensor6.cuh"
-#endif
 #include "pq_tensor.cuh"
 
 bool shape_ok(mevi_ctx* ctx, int d, int M, int K, int metric) {
@@ -342,9 +251,6 @@ bool shape_ok(mevi_ctx* ctx, int d, int M, int K, int metric) {
   if (NT > 128 || NT % 16 != 0) return false;
   return metric == MEVI_METRIC_L2 || metric == MEVI_METRIC_IP;
 }
-// generation 6 needs one 32-candidate block per level and a refinement dot product whose fp32 error stays below U_REL:
-// (d/128 + 8) roundings per element (four FMA chains per lane, two combining adds, five butterfly steps, the product)
-bool v6_ok(int d, int M, int K) { return M >= 2 && K == 32 && d % 128 == 0 && d / 128 + 8 <= 32; }
 
 }  // namespace
 
@@ -363,7 +269,7 @@ bool mevi_rq_tensor_supported(mevi_ctx* ctx, int d, int M, int K, int metric) {
 
 int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
                           int32_t* codes, int64_t codes_stride, float* residual, int64_t* stats, double* inertia,
-                          cudaStream_t st) {
+                          const float* pq_codebook, const KmeansFusedPass* km_fused, cudaStream_t st) {
   if (!mevi_rq_tensor_supported(ctx, d, M, K, metric))
     return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "tensor RQ path unsupported for d=%d M=%d K=%d", d, M, K);
   MEVI_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(X) & 15) == 0 && (reinterpret_cast<uintptr_t>(cb) & 15) == 0,
@@ -374,43 +280,29 @@ int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const
   const int NT = M * K, N1 = 2 * NT, nchunks = d / KC32;
   int gram_floats = 0;
   for (int j = 1; j < M; ++j) gram_floats += j * K * K;
-  // ---- scratch: [consts | absmax2 | work_count | refine_count | cn2 | cnorm | e1 | lvl | cl | ea1 | ea2 | gram | Bimg]
+  // ---- scratch: [consts | absmax2 | work_count | cn2 | cnorm | e1 | lvl | gram | Bimg]
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-  const size_t o_consts = take(C_NUM * 4), o_abs = take(8), o_cnt = take(8), o_ref = take(8), o_cn2 = take(NT * 4),
-               o_cnorm = take(NT * 4), o_e1 = take(NT * 4), o_lvl = take(8 * 4 * 4), o_cl = take(NT * 4), o_ea1 = take(NT * 4),
-               o_ea2 = take(NT * 4), o_gram = take((size_t)(gram_floats ? gram_floats : 1) * 4),
+  const size_t o_consts = take(C_NUM * 4), o_abs = take(8), o_cnt = take(8), o_cn2 = take(NT * 4),
+               o_cnorm = take(NT * 4), o_e1 = take(NT * 4), o_lvl = take(8 * 4 * 4),
+               o_gram = take((size_t)(gram_floats ? gram_floats : 1) * 4),
                o_bimg = take((size_t)nchunks * N1 * KC32 * 2 + 1024);
   char* ws = (char*)mevi_ws(ctx, WS_RQ_PREP, off);
   if (!ws) return MEVI_ERR_NOMEM;
   float* consts = (float*)(ws + o_consts);
   unsigned* absmax2 = (unsigned*)(ws + o_abs);
   unsigned long long* work_count = (unsigned long long*)(ws + o_cnt);
-  unsigned long long* refine_count = (unsigned long long*)(ws + o_ref);
   float* cn2 = (float*)(ws + o_cn2);
   float* cnorm = (float*)(ws + o_cnorm);
   float* lvl = (float*)(ws + o_lvl);
   float* e1 = (float*)(ws + o_e1);
-  float* cl = (float*)(ws + o_cl);
-  float* ea1 = (float*)(ws + o_ea1);
-  float* ea2 = (float*)(ws + o_ea2);
   float* gram = (float*)(ws + o_gram);
   __half* Bimg = (__half*)(ws + o_bimg);
   int32_t* work = (int32_t*)mevi_ws(ctx, WS_RQ_WORK, (size_t)n * 8);
   if (!work) return MEVI_ERR_NOMEM;
   int* err_flag = ctx->dev_err + MEVI_ERRSLOT_RQ;
 
-  const char* ver = getenv("MEVI_RQ_KERNEL");
-  // MEVI_RQ_KERNEL=6 selects generation 6 for the shapes it takes (bit-identical codes; see DESIGN.md for why it is
-  // not the default yet: its in-epilogue refinement is bound by memory latency under the streaming load)
-#ifdef MEVI_WITH_GEN6
-  const bool use_v6 = v6_ok(d, M, K) && ver && atoi(ver) == 6;
-#else
-  const bool use_v6 = false;
-  (void)ver;
-#endif
-
-  MEVI_CUDA(ctx, cudaMemsetAsync(ws + o_abs, 0, o_cn2 - o_abs, st));  // absmax2, work count, refine count
+  MEVI_CUDA(ctx, cudaMemsetAsync(ws + o_abs, 0, o_cn2 - o_abs, st));  // absmax2, work count
   absmax_kernel<<<32, 256, 0, st>>>(cb, (int64_t)M * K, d, 1, absmax2);
   const int64_t sample_rows = 2048;
   const int64_t row_step = n > sample_rows ? n / sample_rows : 1;
@@ -420,118 +312,45 @@ int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const
   cnorm_kernel<<<(NT + 7) / 8, 256, 0, st>>>(cb, M * K, d, NT, cn2, cnorm);
   if (gram_floats) gram_kernel<<<(gram_floats + 7) / 8, 256, 0, st>>>(cb, M, K, d, gram, gram_floats);
   level_consts_kernel<<<M, 32, 0, st>>>(cnorm, cn2, gram, M, K, metric, consts, e1, lvl);
-  if (use_v6) {
-    clo_norm_kernel<<<(NT + 7) / 8, 256, 0, st>>>(cb, M * K, d, NT, consts, cl);
-    loose_consts_kernel<<<1, 128, 0, st>>>(cnorm, cl, NT, metric, ea1, ea2);
-  }
   MEVI_CUDA(ctx, cudaGetLastError());
-  MEVI_COUNT_LAUNCH(ctx, (gram_floats ? 7 : 6) + (use_v6 ? 2 : 0));
+  MEVI_COUNT_LAUNCH(ctx, gram_floats ? 7 : 6);
 
   Params p;
   p.X = X; p.n = n; p.d = d; p.nchunks = nchunks; p.M = M; p.K = K; p.NT = NT; p.N1 = N1; p.metric = metric;
-  p.cb = cb; p.Bimg = Bimg; p.cn2 = cn2; p.e1 = e1; p.lvl = lvl; p.gram = gram; p.consts = consts; p.gram_floats = gram_floats;
-  p.ea1 = ea1; p.ea2 = ea2;
+  p.Bimg = Bimg; p.cn2 = cn2; p.e1 = e1; p.lvl = lvl; p.gram = gram; p.consts = consts; p.gram_floats = gram_floats;
   p.codes = codes; p.codes_stride = codes_stride;
-  p.work_rows = work; p.work_levels = work + n; p.work_count = work_count; p.refine_count = refine_count;
+  p.work_rows = work; p.work_levels = work + n; p.work_count = work_count;
   p.inertia = inertia; p.err_flag = err_flag;
   p.prev = nullptr; p.prev_stride = 0; p.part_sums = nullptr; p.part_counts = nullptr;
-  p.open_rows = nullptr; p.open_meta = nullptr; p.open_t1 = nullptr; p.open_count = nullptr; p.open_cap = 0;
-  {
-    const char* dbg = getenv("MEVI_RQ_DEBUG");
-    p.debug = dbg ? atoi(dbg) : 0;
-  }
-  p.trace = nullptr;
-  const char* trace_path = getenv("MEVI_RQ_TRACE");
-  if (trace_path && *trace_path) {
-    MEVI_CUDA(ctx, cudaMalloc(&p.trace, sizeof(unsigned long long) * (TRACE_SLOTS * TRACE_WARPS + 4)));
-    MEVI_CUDA(ctx, cudaMemsetAsync(p.trace, 0, sizeof(unsigned long long) * (TRACE_SLOTS * TRACE_WARPS + 4), st));
-  }
   CUtensorMap tmap;
-#ifdef MEVI_WITH_GEN6
-  if (use_v6) {
-    int trc = make_x_tensormap(ctx, X, n, d, v6::TM6, &tmap);
-    if (trc != MEVI_OK) return trc;
-    p.n_tiles = (n + v6::TM6 - 1) / v6::TM6;
-    const size_t smem6 = (size_t)v6::smem6_layout(M, NT).total + 1024;
-    const int grid6 = (int)(p.n_tiles < ctx->sm_count ? p.n_tiles : ctx->sm_count);
-    // two-kernel form (default for generation 6; MEVI_RQ_REFINE=inline keeps the refinement inside the epilogue): the open
-    // list holds up to a quarter of the rows (11-12 % are open on N(0,1) data; overflow goes to the exact kernel)
-    const char* rmode = getenv("MEVI_RQ_REFINE");
-    const bool two_kernel = !(rmode && rmode[0] == 'i') && d <= 1024;
-    if (two_kernel) {
-      const int64_t cap = n / 4 + 1024;
-      size_t ooff = 0;
-      auto otake = [&](size_t bytes) { size_t o = ooff; ooff = (ooff + bytes + 255) & ~size_t(255); return o; };
-      const size_t o_cnt2 = otake(8), o_rows = otake((size_t)cap * 4), o_meta = otake((size_t)cap * 16), o_t1 = otake((size_t)cap * M * 32 * 4);
-      char* ows = (char*)mevi_ws(ctx, WS_RQ_OPEN, ooff);
-      if (!ows) return MEVI_ERR_NOMEM;
-      p.open_count = (unsigned long long*)(ows + o_cnt2);
-      p.open_rows = (int32_t*)(ows + o_rows);
-      p.open_meta = (int4*)(ows + o_meta);
-      p.open_t1 = (float*)(ows + o_t1);
-      p.open_cap = cap;
-      MEVI_CUDA(ctx, cudaMemsetAsync(p.open_count, 0, 8, st));
-    }
-    int gram_pad6 = 0;
-    for (int j = 1; j < M; ++j) gram_pad6 += j * 32 * 33;
-    const size_t smem_ref = (size_t)(gram_pad6 + 4 * NT + 16) * 4 + 64;
-#define MEVI_LAUNCH_RQ_TENSOR6(MM)                                                                                          \
-  do {                                                                                                                      \
-    MEVI_CUDA(ctx, cudaFuncSetAttribute(v6::rq_tensor6_kernel<MM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem6)); \
-    v6::rq_tensor6_kernel<MM><<<grid6, v6::THREADS6, smem6, st>>>(p, tmap);                                                 \
-    if (two_kernel && !(p.debug & 256)) {                                                                                   \
-      v6::rq_refine6_kernel<MM><<<ctx->sm_count * 8, 256, smem_ref, st>>>(p);                                               \
-      MEVI_COUNT_LAUNCH(ctx, 1);                                                                                            \
-    }                                                                                                                       \
-  } while (0)
-    switch (M) {
-      case 2: MEVI_LAUNCH_RQ_TENSOR6(2); break;
-      case 3: MEVI_LAUNCH_RQ_TENSOR6(3); break;
-      default: MEVI_LAUNCH_RQ_TENSOR6(4); break;
-    }
-#undef MEVI_LAUNCH_RQ_TENSOR6
-  } else
-#endif
-  {
-    int trc = make_x_tensormap(ctx, X, n, d, v4::TM4, &tmap);
-    if (trc != MEVI_OK) return trc;
-    p.n_tiles = (n + v4::TM4 - 1) / v4::TM4;
-    const size_t smem4 = (size_t)v4::smem4_layout(M, K, NT).total + 1024;
-    const int grid4 = (int)(p.n_tiles < ctx->sm_count ? p.n_tiles : ctx->sm_count);
+  int trc = make_x_tensormap(ctx, X, n, d, v4::TM4, &tmap);
+  if (trc != MEVI_OK) return trc;
+  p.n_tiles = (n + v4::TM4 - 1) / v4::TM4;
+  const size_t smem4 = (size_t)v4::smem4_layout(M, K, NT).total + 1024;
+  const int grid4 = (int)(p.n_tiles < ctx->sm_count ? p.n_tiles : ctx->sm_count);
 #define MEVI_LAUNCH_RQ_TENSOR4(MM)                                                                                          \
   do {                                                                                                                      \
     MEVI_CUDA(ctx, cudaFuncSetAttribute(v4::rq_tensor4_kernel<MM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4)); \
     v4::rq_tensor4_kernel<MM, false><<<grid4, v4::THREADS4, smem4, st>>>(p, tmap);                                          \
   } while (0)
-    if (ctx->km_prev != nullptr && M == 1) {
-      // fused k-means pass: assignment + accumulation under the previous assignment in one read of the shard
-      if (!mevi_kmeans_fused_supported(ctx, d, K))
-        return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "fused k-means pass unsupported for d=%d K=%d", d, K);
-      p.prev = ctx->km_prev; p.prev_stride = ctx->km_prev_stride;
-      p.part_sums = ctx->km_part_sums; p.part_counts = ctx->km_part_counts;
-      const size_t smem_acc = (size_t)v4::smem4_layout(1, K, NT, K * d).total + 1024;
-      MEVI_CUDA(ctx, cudaFuncSetAttribute(v4::rq_tensor4_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_acc));
-      v4::rq_tensor4_kernel<1, true><<<grid4, v4::THREADS4_ACC, smem_acc, st>>>(p, tmap);
-    } else
-    switch (M) {
-      case 1: MEVI_LAUNCH_RQ_TENSOR4(1); break;
-      case 2: MEVI_LAUNCH_RQ_TENSOR4(2); break;
-      case 3: MEVI_LAUNCH_RQ_TENSOR4(3); break;
-      default: MEVI_LAUNCH_RQ_TENSOR4(4); break;
-    }
+  if (km_fused != nullptr && M == 1) {
+    // fused k-means pass: assignment + accumulation under the previous assignment in one read of the shard
+    if (!mevi_kmeans_fused_supported(ctx, d, K))
+      return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "fused k-means pass unsupported for d=%d K=%d", d, K);
+    p.prev = km_fused->prev; p.prev_stride = km_fused->prev_stride;
+    p.part_sums = km_fused->part_sums; p.part_counts = km_fused->part_counts;
+    const size_t smem_acc = (size_t)v4::smem4_layout(1, K, NT, K * d).total + 1024;
+    MEVI_CUDA(ctx, cudaFuncSetAttribute(v4::rq_tensor4_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_acc));
+    v4::rq_tensor4_kernel<1, true><<<grid4, v4::THREADS4_ACC, smem_acc, st>>>(p, tmap);
+  } else
+  switch (M) {
+    case 1: MEVI_LAUNCH_RQ_TENSOR4(1); break;
+    case 2: MEVI_LAUNCH_RQ_TENSOR4(2); break;
+    case 3: MEVI_LAUNCH_RQ_TENSOR4(3); break;
+    default: MEVI_LAUNCH_RQ_TENSOR4(4); break;
+  }
 #undef MEVI_LAUNCH_RQ_TENSOR4
-  }
   MEVI_CUDA(ctx, cudaGetLastError());
-  if (p.trace) {
-    std::vector<unsigned long long> host((size_t)TRACE_SLOTS * TRACE_WARPS + 4);
-    MEVI_CUDA(ctx, cudaStreamSynchronize(st));
-    MEVI_CUDA(ctx, cudaMemcpy(host.data(), p.trace, host.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    cudaFree(p.trace);
-    if (FILE* f = fopen(trace_path, "wb")) {
-      fwrite(host.data(), sizeof(unsigned long long), host.size(), f);
-      fclose(f);
-    }
-  }
   poison_codes_kernel<<<ctx->sm_count, 256, 0, st>>>(err_flag, codes, n, codes_stride, M);
   MEVI_COUNT_LAUNCH(ctx, 2);
   if (int rc = mevi_publish_errors(ctx, st)) return rc;
@@ -540,15 +359,15 @@ int mevi_rq_tensor_assign(mevi_ctx* ctx, const float* X, int64_t n, int d, const
   // is a PQ encode running on a block-padded codebook - the sub-vector kernel, so that flagged rows get exactly the
   // codes mevi_pq_encode's CUDA-core path gives them
   int rc;
-  if (ctx->pq_fix_codebook != nullptr && codes_stride == M)
-    rc = mevi_pq_fix_launch(ctx, X, n, d, ctx->pq_fix_codebook, M, K, metric, codes, work,
+  if (pq_codebook != nullptr && codes_stride == M)
+    rc = mevi_pq_fix_launch(ctx, X, n, d, pq_codebook, M, K, metric, codes, work,
                             reinterpret_cast<const int64_t*>(work_count), st);
   else
     rc = mevi_rq_exact_launch(ctx, X, n, d, cb, M, K, metric, codes, codes_stride, nullptr, work, work + n,
                               reinterpret_cast<const int64_t*>(work_count), n, nullptr, st);
   if (rc != MEVI_OK) return rc;
   if (stats) {
-    finish_stats_kernel<<<1, 32, 0, st>>>(work_count, refine_count, n, stats);
+    finish_stats_kernel<<<1, 32, 0, st>>>(work_count, n, stats);
     MEVI_COUNT_LAUNCH(ctx, 1);
   }
   if (residual) {
@@ -568,7 +387,7 @@ bool mevi_pq_tensor_supported(mevi_ctx* ctx, int64_t n, int d, int M, int K, int
 }
 
 int mevi_pq_tensor_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const float* cb, int M, int K, int metric,
-                          int32_t* codes, int64_t* stats, cudaStream_t st) {
+                          int32_t* codes, cudaStream_t st) {
   if (!mevi_pq_tensor_supported(ctx, n, d, M, K, metric))
     return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "tensor PQ path unsupported for d=%d M=%d K=%d", d, M, K);
   if (n <= 0) return MEVI_OK;
@@ -607,16 +426,6 @@ int mevi_pq_tensor_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const
   p.codes = codes; p.pairs = pairs; p.pair_count = pair_count; p.pair_cap = cap; p.overflow = overflow;
   p.err_flag = err_flag;
   p.n_tiles = (n + pq256::TMQ - 1) / pq256::TMQ;
-  {
-    const char* dbg = getenv("MEVI_RQ_DEBUG");
-    p.debug = dbg ? atoi(dbg) : 0;
-  }
-  p.trace = nullptr;
-  const char* pq_trace = getenv("MEVI_PQ_TRACE");
-  if (pq_trace && *pq_trace) {
-    MEVI_CUDA(ctx, cudaMalloc(&p.trace, sizeof(unsigned long long) * pq256::TRQ_SLOTS * pq256::TRQ_WARPS));
-    MEVI_CUDA(ctx, cudaMemsetAsync(p.trace, 0, sizeof(unsigned long long) * pq256::TRQ_SLOTS * pq256::TRQ_WARPS, st));
-  }
   CUtensorMap tmap;
   // 128-byte L2 promotion: a pass reads 384-byte row pieces, 256-byte promotion would fetch 512
   int trc = make_x_tensormap(ctx, X, n, d, pq256::TMQ, &tmap, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, ds);
@@ -631,25 +440,8 @@ int mevi_pq_tensor_encode(mevi_ctx* ctx, const float* X, int64_t n, int d, const
     pq256::pq_tensor_kernel<24><<<grid, pq256::THREADSQ, smem, st>>>(p, tmap);
   }
   MEVI_CUDA(ctx, cudaGetLastError());
-  if (p.trace) {
-    std::vector<unsigned long long> host((size_t)pq256::TRQ_SLOTS * pq256::TRQ_WARPS);
-    MEVI_CUDA(ctx, cudaStreamSynchronize(st));
-    MEVI_CUDA(ctx, cudaMemcpy(host.data(), p.trace, host.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    cudaFree(p.trace);
-    if (FILE* f = fopen(pq_trace, "wb")) {
-      fwrite(host.data(), sizeof(unsigned long long), host.size(), f);
-      fclose(f);
-    }
-  }
   poison_codes_kernel<<<ctx->sm_count, 256, 0, st>>>(err_flag, codes, n, M, M);
   MEVI_COUNT_LAUNCH(ctx, 7);
   if (int rc = mevi_publish_errors(ctx, st)) return rc;
-  int rc = mevi_pq_fix_pairs_launch(ctx, X, n, d, cb, M, K, metric, codes, pairs, pair_count, cap, overflow, st);
-  if (rc != MEVI_OK) return rc;
-  if (stats) {  // stats[0] += undecided (row, sub-vector) pairs, stats[1] += rows
-    finish_stats_kernel<<<1, 32, 0, st>>>(pair_count, pair_count, n, stats);
-    MEVI_COUNT_LAUNCH(ctx, 1);
-  }
-  MEVI_CUDA(ctx, cudaGetLastError());
-  return MEVI_OK;
+  return mevi_pq_fix_pairs_launch(ctx, X, n, d, cb, M, K, metric, codes, pairs, pair_count, cap, overflow, st);
 }

@@ -89,15 +89,12 @@ __device__ __forceinline__ void converter_loop4(const Params& p, uint8_t* sX, fl
   const uint32_t t_lane = tmem_base + ((uint32_t)((cw & 3) * 32) << 16) + A_COL0 + (uint32_t)half * 32u;
   float2 norm2 = make_float2(0.f, 0.f);  // (even, odd) partial sums of the squared row norm
   const float2 sx2 = make_float2(sx, sx);
-  uint32_t xs = 0, xph = 0, as = 0, aph = 0, it = 0, pend_stage = 0, tix = 0;
-  const int warp = cw + CONV_WARP0;
+  uint32_t xs = 0, xph = 0, as = 0, aph = 0, it = 0, pend_stage = 0;
   bool pending = false;
   for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
     for (int c = 0; c < nchunks; ++c) {
       if (!ptx::mbar_wait(&x_full[xs], xph)) { atomicExch(p.err_flag, 4); return; }
-      trace_ev(p, warp, lane, tix, it, c, 0);  // X stage landed
       if (!ptx::mbar_wait_backoff(&a_empty[as], aph ^ 1, 32)) { atomicExch(p.err_flag, 4); return; }
-      trace_ev(p, warp, lane, tix, it, c, 1);  // operand stage free
       ptx::tc_fence_after_sync();
       uint32_t hi[16], lo[16];
 #pragma unroll
@@ -129,7 +126,6 @@ __device__ __forceinline__ void converter_loop4(const Params& p, uint8_t* sX, fl
       // the stores consumed every value loaded from the X stage: hand it back to the TMA producer
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(&x_empty[xs]);
-      trace_ev(p, warp, lane, tix, it, c, 2);  // converted, stores issued
       pending = true;
       pend_stage = as;
       if (++xs == NSX) { xs = 0; xph ^= 1; }
@@ -230,19 +226,17 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
   __syncthreads();
   ptx::tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_holder;
-  trace_clock(p, 0);
 
   // The three control warps walk their loops with all 32 lanes (operands stay warp-uniform) and issue from one
   // elected lane: `if (lane == 0)` would wrap every TMA / tcgen05 instruction in an R2UR waterfall loop.
   if (warp == 0) {
-    uint32_t s = 0, ph = 0, tix = 0, it = 0;
-    for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
+    uint32_t s = 0, ph = 0;
+    for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
       for (int c = 0; c < nchunks; ++c) {
         if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait_backoff(&x_empty[s], ph ^ 1, 32))) {
           if (lane == 0) atomicExch(p.err_flag, 1);
           return;
         }
-        trace_ev(p, warp, lane, tix, it, c, 0);
         if (ptx::elect_one()) {
           ptx::mbar_arrive_expect_tx(&x_full[s], X_STAGE4);
           ptx::tma_load_2d(sX + (size_t)s * X_STAGE4, &tmap, c * KC4, (int)(tile * TM4), &x_full[s]);
@@ -252,19 +246,16 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
       }
     }
   } else if (warp == 3) {
-    uint32_t s = 0, ph = 0, tix = 0, it = 0;
-    for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
+    uint32_t s = 0, ph = 0;
+    for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
       for (int c = 0; c < nchunks; ++c) {
         if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait_backoff(&a_empty[s], ph ^ 1, 32))) {
           if (lane == 0) atomicExch(p.err_flag, 7);
           return;
         }
-        trace_ev(p, warp, lane, tix, it, c, 0);
         if (ptx::elect_one()) {
-          const bool twice = (p.debug & 16) != 0;  // experiment: what would twice the codebook traffic cost?
-          ptx::mbar_arrive_expect_tx(&b_full[s], twice ? 2 * b_stage_bytes : b_stage_bytes);
+          ptx::mbar_arrive_expect_tx(&b_full[s], b_stage_bytes);
           ptx::bulk_g2s(sB + (size_t)s * b_stage_bytes, p.Bimg + (size_t)c * (2 * NT) * KC4, b_stage_bytes, &b_full[s]);
-          if (twice) ptx::bulk_g2s(sB + (size_t)s * b_stage_bytes, p.Bimg + (size_t)c * (2 * NT) * KC4, b_stage_bytes, &b_full[s]);
         }
         __syncwarp();
         if (++s == NSB4) { s = 0; ph ^= 1; }
@@ -277,7 +268,7 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
     const int h = warp - 1;
     const uint32_t idesc = ptx::umma_idesc_f16_m128((uint32_t)NT);
     const uint32_t d_tmem = tmem_base + h * 128;
-    uint32_t as = 0, aph = 0, it = 0, tix = 0;
+    uint32_t as = 0, aph = 0, it = 0;
     for (int64_t tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
       // single accumulator buffer: the previous tile's epilogue must have drained it
       if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait(acc_empty, (it & 1) ^ 1))) {
@@ -285,31 +276,25 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
         return;
       }
       ptx::tc_fence_after_sync();
-      trace_ev(p, warp, lane, tix, it, 255, 3);  // accumulator free
       for (int c = 0; c < nchunks; ++c) {
         if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait(&a_full[as], aph))) {
           if (lane == 0) atomicExch(p.err_flag, 3);
           return;
         }
-        trace_ev(p, warp, lane, tix, it, c, 0);  // operand stage full
         if (!__all_sync(MEVI_FULL_MASK, ptx::mbar_wait(&b_full[as], aph))) {
           if (lane == 0) atomicExch(p.err_flag, 3);
           return;
         }
-        trace_ev(p, warp, lane, tix, it, c, 1);  // codebook stage full
         ptx::tc_fence_after_sync();
         const uint32_t b_hi = ptx::smem_u32(sB + (size_t)as * b_stage_bytes);
         const uint32_t b_lo = b_hi + (uint32_t)NT * 64u;
         if (ptx::elect_one()) {
-          if (!(p.debug & 2)) {
-            const uint32_t a_hi = tmem_base + A_COL0 + as * 64 + h * 32, a_lo = a_hi + 16;
+          const uint32_t a_hi = tmem_base + A_COL0 + as * 64 + h * 32, a_lo = a_hi + 16;
 #pragma unroll
-            for (int ks = 0; ks < KC4 / 16; ++ks) {
-              ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, (c | ks) != 0 ? 1u : 0u);
-              if (p.debug & 32) continue;  // experiment: hi.hi only (a third of the tensor work; results are approximate)
-              ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_lo + ks * 32), idesc, 1u);
-              ptx::umma_f16_ts(d_tmem, a_lo + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, 1u);
-            }
+          for (int ks = 0; ks < KC4 / 16; ++ks) {
+            ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, (c | ks) != 0 ? 1u : 0u);
+            ptx::umma_f16_ts(d_tmem, a_hi + ks * 8, ptx::umma_desc_sw64(b_lo + ks * 32), idesc, 1u);
+            ptx::umma_f16_ts(d_tmem, a_lo + ks * 8, ptx::umma_desc_sw64(b_hi + ks * 32), idesc, 1u);
           }
           // the operand (TMEM) and codebook (smem) rings advance in lockstep: converters and the codebook producer
           // both wait on a_empty[as], which completes when BOTH MMA warps have committed
@@ -317,7 +302,6 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
           if (c == nchunks - 1) ptx::umma_commit(acc_full);
         }
         __syncwarp();
-        trace_ev(p, warp, lane, tix, it, c, 2);  // issued + committed
         if (++as == NSA4) { as = 0; aph ^= 1; }
       }
     }
@@ -444,7 +428,7 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
         // sum in the staging buffer of this chunk's parity.
         const uint32_t stage_u32 = ptx::smem_u32(sX) + xs * X_STAGE4;
         float4* part = sPart + (c & 1) * MAX_STEPS4 * 8;
-        const int nsteps = (p.debug & 128) ? 0 : step0[K];
+        const int nsteps = step0[K];
         for (int base = aw * 4; base < nsteps; base += 4 * ACC_WARPS) {
           // four steps per warp at a time, one per group of 8 lanes: no cross-lane reduction, 4 independent row streams.
           // The sorter left every step's 16 row offsets in a table (0xFFFF = past the end of the list -> zero line).
@@ -507,12 +491,11 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
     const float m2inv = (p.metric == MEVI_METRIC_L2 ? -2.f : -1.f) * p.consts[C_INV];
     const bool l2 = p.metric == MEVI_METRIC_L2;
     double inertia_acc = 0.0;
-    uint32_t it = 0, tix = 0;
+    uint32_t it = 0;
     bool ok = true;
     for (int64_t tile = blockIdx.x; tile < p.n_tiles && ok; tile += gridDim.x, ++it) {
       if (!ptx::mbar_wait_backoff(acc_full, it & 1, 64) || !ptx::mbar_wait_backoff(&st_full[it & 1], (it >> 1) & 1, 32)) { atomicExch(p.err_flag, 6); ok = false; break; }
       ptx::tc_fence_after_sync();
-      trace_ev(p, warp, lane, tix, it, 255, 0);  // accumulators ready
       // (fused k-means variant: 4 epilogue warps, each takes its lane quarter of BOTH halves)
       for (int h = ACC ? 0 : (ew >> 2); h < (ACC ? 2 : (ew >> 2) + 1); ++h) {
         const int q = ew & 3;  // 32-lane quarter of TMEM (== warp % 4)
@@ -528,7 +511,6 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
         for (int j = 0; j < M; ++j) code[j] = 0;
 #pragma unroll
         for (int j = 0; j < M; ++j) {
-          if (p.debug & 4) break;
           const float* gj = sGram + (j * (j - 1) / 2) * K * (K + 1);
           const float* grow[M > 1 ? M - 1 : 1];
 #pragma unroll
@@ -589,7 +571,6 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
       }
       ptx::tc_fence_before_sync();
       __syncwarp();
-      trace_ev(p, warp, lane, tix, it, 255, 1);  // accumulators drained
       if (lane == 0) ptx::mbar_arrive(acc_empty);
     }
     if (p.inertia) {
@@ -601,7 +582,6 @@ rq_tensor4_kernel(Params p, const __grid_constant__ CUtensorMap tmap) {
 
   ptx::tc_fence_before_sync();
   __syncthreads();
-  trace_clock(p, 1);
   if (warp == 2) ptx::tmem_dealloc(tmem_base, TMEM_COLS);
   if (ACC) {  // per-CTA partials; reduced in CTA order by kmeans_reduce_partials_kernel (deterministic)
     const int64_t kd = (int64_t)K * p.d;

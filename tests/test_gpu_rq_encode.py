@@ -178,27 +178,3 @@ def test_config_i_100k_golden_codes():
         codes, stats = c.rq_encode(dev(X), dev(cb), mode=mode, return_stats=True)
         rep = _check(X, cb, codes.cpu().numpy(), want)
         print("gauss100k", mode, "mismatch", rep["n_mismatch"], "ties", rep["n_ties"], "stats", stats.tolist()[:3])
-
-
-def test_generation6_kernel_matches_the_exact_kernel(monkeypatch, gauss):
-    """The hi.hi prefilter + refinement kernel (csrc/experiments/rq_tensor6.cuh; measured slower than generation 4 and not
-    part of the shipped library - `make -C mevi_b200/csrc GEN6=1` and MEVI_TEST_GEN6=1 to run this): same codes as the
-    direct kernel."""
-    import os
-
-    if os.environ.get("MEVI_TEST_GEN6", "0") == "0":
-        pytest.skip("generation 6 is an experiment outside the shipped library (build with GEN6=1, set MEVI_TEST_GEN6=1)")
-    c = ctx()
-    rs = np.random.RandomState(3)
-    X = rs.standard_normal((50000, 768)).astype(np.float32)
-    X[::7] *= 3.0
-    X[5] = 0.0
-    for M in (2, 3, 4):
-        cb = gauss.codebook[:M].copy()
-        want = c.rq_encode(dev(X), dev(cb), mode="exact").cpu().numpy()
-        monkeypatch.setenv("MEVI_RQ_KERNEL", "6")
-        got, stats = c.rq_encode(dev(X), dev(cb), mode="tensor", return_stats=True)
-        monkeypatch.delenv("MEVI_RQ_KERNEL")
-        c.check()
-        assert int(stats[2].item()) > 0  # the refinement path ran
-        _check(X, cb, got.cpu().numpy(), want)

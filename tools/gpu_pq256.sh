@@ -37,9 +37,6 @@ def run(tag, reps=5):
     t.record(); torch.cuda.synchronize(); ms = s.elapsed_time(t) / reps
     print(f"{tag:40s} {ms:8.3f} ms  {n*3072/ms/1e6:7.0f} GB/s  frac {n*3072/ms/1e6/6541.8:.3f}", flush=True)
 run("pq 24x256 tensor")
-for dbg, name in ((2, "no MMA"), (4, "no epilogue reduction"), (6, "no MMA, no epilogue"), (30, "handshakes only")):
-    os.environ["MEVI_RQ_DEBUG"] = str(dbg); run(f"debug={dbg} ({name})", reps=3)
-os.environ["MEVI_RQ_DEBUG"] = "0"
 cb24 = torch.randn((32, 256, 24), device="cuda"); cb32 = cb; cb = cb24; run("pq 32x256 (width 24) tensor"); cb = cb32
 a = ctx.pq_encode(X[:200000], cb); os.environ["MEVI_PQ_TENSOR"] = "0"; e = ctx.pq_encode(X[:200000], cb)
 print("mismatch on 200k of the timed matrix:", int((a != e).sum()))
