@@ -185,6 +185,14 @@ int mevi_build_inverted_lists(mevi_ctx* ctx, const int32_t* codes, int64_t n, in
  *   leaf_keys, -1 when no document carries it or a code is outside [0, K).                                        */
 int mevi_leaf_lookup(mevi_ctx* ctx, const int64_t* leaves, int64_t n_pairs, int M, int K, const int64_t* leaf_keys,
                      int64_t n_leaves, int32_t* leaf_index, void* stream);
+/* Occurrence table of inverted lists in which a document may be listed under several leaves (`--doc_multiclus > 1`):
+ * a device sort of (document, CSR position), grouped by document.  *max_occ_host = C, the largest number of positions
+ * of any document (0 when n == 0).  With occ_leaves != NULL ([n, width] int32, width >= C - 1) row p receives the CSR
+ * leaf indices of the other positions of the document at position p, in ascending position order, -1 padded; a
+ * position p' < p in the same leaf (a leaf listing the document twice) is written as -2 - leaf.
+ * Synchronises `stream`.  MEVI_ERR_INVALID when width < C - 1.                                                     */
+int mevi_occurrence_table(mevi_ctx* ctx, const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
+                          int64_t n, int width, int32_t* occ_leaves, int32_t* max_occ_host, void* stream);
 
 /* ---- cluster-restricted re-rank ----------------------------------------- *
  * replaces: MEVI/main_models.py:3915-4014 (per query: leaves -> candidate rows
@@ -213,6 +221,25 @@ int mevi_cluster_rerank_prefix(mevi_ctx* ctx, const float* Q, int nq, const floa
                                const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
                                const int32_t* query_leaves, int L, int k, int64_t max_rows, float* scores, int64_t* ids,
                                int32_t* n_candidates, void* stream);
+
+/* mevi_cluster_rerank (leaf-ordered layout) for an index built with `--doc_multiclus > 1`, where a document is listed
+ * under up to C leaves: one entry per document, like main_models.py:3998-4011 followed by the sort and the
+ * `[:save_hard_neg]` truncation.  For a query and a document, let c be the number of positions of the query's leaf list
+ * whose leaf lists the document (a leaf repeated in the list counts once per position, a leaf listing the document
+ * twice counts twice: the reference's concatenation) and s its fp32 score (the same
+ * at every position).  Its score is s for aggr = MEVI_MULTICLUS_MAX, and the fp32 fold ((0 + s) + s) + ... of c terms
+ * for MEVI_MULTICLUS_ADD.  Output as mevi_cluster_rerank: the k best distinct documents by (score desc, id asc);
+ * n_candidates counts occurrences (the reference's cur_ndoc).
+ *   occ_leaves [n, C-1] int32 from mevi_occurrence_table (NULL when C == 1): per CSR position, the CSR leaf indices of
+ *              the document's other positions, -1 padded.  16-byte aligned; the kernel copies it in 16-byte
+ *              aligned pieces, so the allocation must extend to the next multiple of 16 bytes past n*(C-1)*4.
+ * MEVI_ERR_UNSUPPORTED for C > 16, and for shapes the streaming kernel does not take.                              */
+#define MEVI_MULTICLUS_ADD 0
+#define MEVI_MULTICLUS_MAX 1
+int mevi_cluster_rerank_multiclus(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int64_t n, int d,
+                                  const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
+                                  const int32_t* occ_leaves, int C, const int32_t* query_leaves, int L, int k, int aggr,
+                                  int64_t id_base, float* scores, int64_t* ids, int32_t* n_candidates, void* stream);
 
 /* The same loop keeping EVERY candidate (the shipped recipe runs `--save_hard_neg 8841823`: main_models.py:4012-4014,
  * 4046-4053 write all candidates, sorted): leaf-ordered layout only.  Candidate number pos of query q, in the

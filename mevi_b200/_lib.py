@@ -19,6 +19,7 @@ METRIC_L2, METRIC_IP = 0, 1
 MODE_AUTO, MODE_EXACT, MODE_TENSOR = 0, 1, 2
 _MODES = {"auto": MODE_AUTO, "exact": MODE_EXACT, "tensor": MODE_TENSOR}
 _METRICS = {"l2": METRIC_L2, "ip": METRIC_IP}
+_MULTICLUS_AGGR = {"add": 0, "max": 1}  # MEVI_MULTICLUS_ADD / _MAX
 
 # every symbol include/mevi_b200.h declares: (restype, argtypes)
 _vp, _i, _i64, _f, _d = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double
@@ -41,7 +42,10 @@ SYMBOLS = {
     "mevi_rq_beam_search": (_i, [_vp, _vp, _i64, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "mevi_build_inverted_lists": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp]),
     "mevi_leaf_lookup": (_i, [_vp, _vp, _i64, _i, _i, _vp, _i64, _vp, _vp]),
+    "mevi_occurrence_table": (_i, [_vp, _vp, _i64, _vp, _i64, _i, _vp, C.POINTER(C.c_int32), _vp]),
     "mevi_cluster_rerank": (_i, [_vp, _vp, _i, _vp, _i64, _i, _i, _vp, _i64, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp]),
+    "mevi_cluster_rerank_multiclus": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _i64, _vp, _vp, _i, _vp, _i, _i, _i, _i64, _vp, _vp,
+                                           _vp, _vp]),
     "mevi_cluster_rerank_prefix": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _i64, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp]),
     "mevi_cluster_rerank_all": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _i64, _vp, _vp, _i, _i64, _vp, _vp, _vp, _vp, _vp]),
     "mevi_rerank_grouped_image": (_i, [_vp, _vp, _i64, _i, _vp, _i64, _vp, C.POINTER(_f), C.POINTER(_f), _vp]),
@@ -422,6 +426,50 @@ class Context:
                                              _ptr(ql), L, int(k), int(id_base), _ptr(scores), _ptr(ids), _ptr(ncand),
                                              self._stream())
             )
+        return scores, ids, ncand
+
+    def occurrence_table(self, leaf_offsets, leaf_docids):
+        """Inverted lists that may list a document under several leaves -> (occ int32 [n, C-1], C): row p holds the CSR
+        leaf indices of the other positions of the document at CSR position p, -1 padded (-2 - leaf for an earlier
+        position in the same leaf); C = the largest number of
+        positions of any document (1 for an empty or single-cluster index)."""
+        import torch
+
+        lo = self._dev(leaf_offsets, torch.int64, "leaf_offsets")
+        ld = self._dev(leaf_docids, torch.int32, "leaf_docids")
+        n = ld.numel()
+        c = C.c_int32(0)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mevi_occurrence_table(self.handle, _ptr(lo), lo.numel() - 1, _ptr(ld), n, 0, None, C.byref(c),
+                                                       self._stream()))
+            n_occ = max(int(c.value), 1)
+            # 16 B of slack: mevi_cluster_rerank_multiclus copies the table in 16-byte aligned pieces
+            occ = torch.empty(n * (n_occ - 1) + 4, dtype=torch.int32, device=ld.device)[: n * (n_occ - 1)].view(n, n_occ - 1)
+            if n_occ > 1:
+                self._check(self.lib.mevi_occurrence_table(self.handle, _ptr(lo), lo.numel() - 1, _ptr(ld), n, n_occ - 1,
+                                                           _ptr(occ), C.byref(c), self._stream()))
+        return occ, n_occ
+
+    def cluster_rerank_multiclus(self, Q, D_leaf, leaf_offsets, leaf_docids, occ, n_occ, query_leaves, k, aggr, id_base=0):
+        """Top-k of a multi-cluster index (`--doc_multiclus > 1`): one entry per document, its score aggregated over the
+        query's leaves that list it (aggr 'add' / 'max'); occ, n_occ from occurrence_table."""
+        import torch
+
+        Q = self._dev(Q, torch.float32, "Q")
+        D = self._dev(D_leaf, torch.float32, "D_leaf")
+        lo = self._dev(leaf_offsets, torch.int64, "leaf_offsets")
+        ld = self._dev(leaf_docids, torch.int32, "leaf_docids")
+        ql = self._dev(query_leaves, torch.int32, "query_leaves")
+        occ = self._dev(occ, torch.int32, "occ")
+        nq, d = Q.shape
+        scores = torch.empty((nq, k), dtype=torch.float32, device=Q.device)
+        ids = torch.empty((nq, k), dtype=torch.int64, device=Q.device)
+        ncand = torch.empty((nq,), dtype=torch.int32, device=Q.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mevi_cluster_rerank_multiclus(
+                self.handle, _ptr(Q), nq, _ptr(D), D.shape[0], d, _ptr(lo), lo.numel() - 1, _ptr(ld),
+                _ptr(occ) if occ.numel() else None, int(n_occ), _ptr(ql), ql.shape[1], int(k), _MULTICLUS_AGGR[aggr],
+                int(id_base), _ptr(scores), _ptr(ids), _ptr(ncand), self._stream()))
         return scores, ids, ncand
 
     def cluster_rerank_all(self, Q, D_leaf, leaf_offsets, leaf_docids, query_leaves, id_base=0):

@@ -205,20 +205,51 @@ constexpr int RS_STAGES = 6;
 constexpr int RS_CONSUMERS = 8; // warps 1..8; warp 0 is the producer
 constexpr int RS_THREADS = 32 * (1 + RS_CONSUMERS);
 constexpr int RS_CHECK = 16;    // stages between compaction checks (<= 128 appends)
+constexpr int RS_OCC_SLOT = 512;  // multi-cluster: the stage's rows of the occurrence table (<= 8 x 15 int32, 16 B aligned)
 
 __device__ __forceinline__ void consumer_bar() { asm volatile("bar.sync 1, %0;" ::"n"(32 * RS_CONSUMERS) : "memory"); }
 
-template <int NCH>
-__global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams p) {
+// --doc_multiclus > 1 (main_models.py:3998-4011): a document listed under several leaves has several CSR positions.
+// occ_leaves [n, C-1] int32 holds, per CSR position, the leaves of the document's OTHER positions (-1 padded; -2 - leaf
+// for an earlier position in the same leaf, when a leaf lists the document more than once).  Per
+// (query, document) exactly one occurrence is kept, the canonical one: the first position of the query's leaf list whose
+// leaf lists the document (and the first CSR position inside that leaf).  It is scored agg(c, s), c = the number of positions of the leaf list that list the document.
+struct MultiClus {
+  const int32_t* occ_leaves;
+  int C;         // largest number of positions of any document (1 <= C <= 16)
+  int aggr;      // MEVI_MULTICLUS_ADD / _MAX
+  int hash_log2; // the per-CTA leaf table has 1 << hash_log2 >= 2L slots
+};
+
+__device__ __forceinline__ int leaf_slot(const int32_t* s_hkey, int leaf, int hash_log2) {
+  const unsigned mask = (1u << hash_log2) - 1u;
+  unsigned h = ((unsigned)leaf * 0x9E3779B1u) >> (32 - hash_log2);
+  for (;;) {  // load factor <= 1/2: a free slot ends every probe sequence
+    const int k = s_hkey[h];
+    if (k == leaf) return (int)h;
+    if (k < 0) return -1;
+    h = (h + 1) & mask;
+  }
+}
+
+template <int NCH, bool MC>
+__device__ __forceinline__ void rerank_stream_body(const RerankParams& p, const MultiClus& mc) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int d = p.d;
   const uint32_t row_bytes = (uint32_t)d * 4u;
   const uint32_t stage_bytes = RS_ROWS * row_bytes;
   unsigned char* s_ring = smem_raw;                                                  // [RS_STAGES][RS_ROWS][d] fp32
-  float* s_score = reinterpret_cast<float*>(s_ring + (size_t)RS_STAGES * stage_bytes);
+  unsigned char* s_occ = s_ring + (size_t)RS_STAGES * stage_bytes;                    // MC: [RS_STAGES][RS_OCC_SLOT]
+  float* s_score = reinterpret_cast<float*>(s_occ + (MC ? RS_STAGES * RS_OCC_SLOT : 0));
   int32_t* s_id = reinterpret_cast<int32_t*>(s_score + p.cap);
   int64_t* s_prefix = reinterpret_cast<int64_t*>(s_id + p.cap);                      // [L+1]
   int64_t* s_leafbeg = s_prefix + (p.L + 1);                                         // [L]
+  // MC: open-addressed table of the query's leaves -> first position in its leaf list, number of positions; and per
+  // position t its leaf's number of positions when t is that leaf's first position, else -1 (a repeated leaf)
+  int32_t* s_hkey = reinterpret_cast<int32_t*>(s_leafbeg + p.L);                     // [1 << hash_log2]
+  int32_t* s_hfirst = s_hkey + (MC ? (1 << mc.hash_log2) : 0);
+  int32_t* s_hmult = s_hfirst + (MC ? (1 << mc.hash_log2) : 0);
+  int32_t* s_own = s_hmult + (MC ? (1 << mc.hash_log2) : 0);                          // [L]
   __shared__ __align__(8) uint64_t full_bar[RS_STAGES];
   __shared__ __align__(8) uint64_t empty_bar[RS_STAGES];
   __shared__ int s_meta_row[RS_STAGES];
@@ -241,6 +272,13 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
     s_leafbeg[t] = b;
     s_prefix[t + 1] = sz;
   }
+  if constexpr (MC) {
+    for (int i = tid; i < (1 << mc.hash_log2); i += RS_THREADS) {
+      s_hkey[i] = -1;
+      s_hfirst[i] = 0x7fffffff;
+      s_hmult[i] = 0;
+    }
+  }
   if (tid == 0) {
     s_prefix[0] = 0;
     s_count = 0;
@@ -252,6 +290,22 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
     ptx::mbar_fence_init();
   }
   __syncthreads();
+  if constexpr (MC) {  // (before the scan below overwrites the leaf sizes)
+    for (int t = tid; t < p.L; t += RS_THREADS) {
+      if (s_prefix[t + 1] == 0) continue;  // no document: never streamed, never a sibling
+      const int leaf = p.query_leaves[(int64_t)q * p.L + t];
+      const unsigned mask = (1u << mc.hash_log2) - 1u;
+      unsigned h = ((unsigned)leaf * 0x9E3779B1u) >> (32 - mc.hash_log2);
+      for (;;) {
+        const int prev = atomicCAS(&s_hkey[h], -1, leaf);
+        if (prev < 0 || prev == leaf) break;
+        h = (h + 1) & mask;
+      }
+      atomicMin(&s_hfirst[h], t);
+      atomicAdd(&s_hmult[h], 1);
+    }
+    __syncthreads();
+  }
   if (tid == 0) {
     int64_t run = 0;
     for (int t = 1; t <= p.L; ++t) {
@@ -260,6 +314,17 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
     }
   }
   __syncthreads();
+  if constexpr (MC) {
+    for (int t = tid; t < p.L; t += RS_THREADS) {
+      int own = -1;
+      if (s_prefix[t + 1] > s_prefix[t]) {
+        const int h = leaf_slot(s_hkey, p.query_leaves[(int64_t)q * p.L + t], mc.hash_log2);
+        if (s_hfirst[h] == t) own = s_hmult[h];
+      }
+      s_own[t] = own;
+    }
+    __syncthreads();
+  }
   int64_t C = s_prefix[p.L];
   if (s == 0 && tid == 0 && p.n_candidates) p.n_candidates[q] = (int32_t)(C > 0x7fffffff ? 0x7fffffff : C);
   if (p.max_rows > 0 && C > p.max_rows) C = p.max_rows;
@@ -279,10 +344,19 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
           const uint32_t st = g % RS_STAGES, ph = (g / RS_STAGES) & 1;
           if (!ptx::mbar_wait(&empty_bar[st], ph ^ 1)) { atomicExch(p.err_flag, 1); ok = false; break; }
           s_meta_row[st] = (int)row;
-          s_meta_n[st] = nrows;
+          s_meta_n[st] = MC ? (nrows | (t << 4)) : nrows;  // MC: the leaf's position in the query's list rides along
           const uint32_t bytes = (uint32_t)nrows * row_bytes;
-          ptx::mbar_arrive_expect_tx(&full_bar[st], bytes);
+          uint32_t occ_bytes = 0;
+          int64_t occ0 = 0;
+          if constexpr (MC) {  // the rows' slice of the occurrence table travels with them, widened to 16 B bounds
+            const int64_t w4 = (int64_t)(mc.C - 1) * 4;
+            occ0 = (row * w4) & ~int64_t(15);
+            occ_bytes = (uint32_t)((((row + nrows) * w4 + 15) & ~int64_t(15)) - occ0);
+          }
+          ptx::mbar_arrive_expect_tx(&full_bar[st], bytes + occ_bytes);
           ptx::bulk_g2s(s_ring + (size_t)st * stage_bytes, p.D + row * d, bytes, &full_bar[st]);
+          if (occ_bytes)
+            ptx::bulk_g2s(s_occ + st * RS_OCC_SLOT, reinterpret_cast<const char*>(mc.occ_leaves) + occ0, occ_bytes, &full_bar[st]);
         }
       }
       // sentinel: tells the consumers the stream has ended
@@ -311,10 +385,19 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
     for (;; ++g) {
       const uint32_t st = g % RS_STAGES, ph = (g / RS_STAGES) & 1;
       if (!ptx::mbar_wait(&full_bar[st], ph)) { atomicExch(p.err_flag, 3); break; }
-      const int nrows = s_meta_n[st];
+      const int meta = s_meta_n[st];
+      const int nrows = MC ? (meta & 15) : meta;
       if (nrows == 0) break;
       if (cw < nrows) {
         const float* src = reinterpret_cast<const float*>(s_ring + (size_t)st * stage_bytes + (size_t)cw * row_bytes);
+        int32_t sib = -1;
+        if constexpr (MC) {
+          if (lane >= 1 && lane < mc.C) {
+            const int64_t w = mc.C - 1, row0 = s_meta_row[st];
+            const int64_t e = (row0 + cw) * w + (lane - 1) - (((row0 * w * 4) & ~int64_t(15)) >> 2);
+            sib = reinterpret_cast<const int32_t*>(s_occ + st * RS_OCC_SLOT)[e];
+          }
+        }
         float acc = 0.f;
 #pragma unroll
         for (int t = 0; t < NCH; ++t) {
@@ -328,7 +411,34 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
           }
         }
         acc = warp_sum(acc);
-        if (lane == 0) {
+        bool keep = true;
+        if constexpr (MC) {
+          // lane 0: this position's own leaf; lanes 1..C-1: the leaves of the document's other positions.  The occurrence
+          // is canonical when no leaf of the document comes earlier in the query's list.
+          const int t = meta >> 4;
+          int mult = 0;
+          bool earlier = false;
+          if (lane == 0) {
+            mult = s_own[t];
+            earlier = mult < 0;
+          } else if (sib <= -2) {  // the document also sits at an earlier position of this same leaf
+            earlier = true;
+          } else if (sib >= 0) {
+            const int h = leaf_slot(s_hkey, sib, mc.hash_log2);
+            if (h >= 0) {
+              mult = s_hmult[h];
+              earlier = s_hfirst[h] < t;
+            }
+          }
+          keep = __ballot_sync(MEVI_FULL_MASK, earlier) == 0u;
+          const int c = __reduce_add_sync(MEVI_FULL_MASK, earlier ? 0 : mult);
+          if (keep && mc.aggr == MEVI_MULTICLUS_ADD) {
+            float a = 0.f;  // the reference's fold: zeros, then += s once per position (main_models.py:4004-4007)
+            for (int i = 0; i < c; ++i) a = __fadd_rn(a, acc);
+            acc = a;
+          }
+        }
+        if (lane == 0 && keep) {
           const float tau = *reinterpret_cast<volatile float*>(&s_tau);
           if (!(acc < tau)) {
             const int slot = atomicAdd(&s_count, 1);
@@ -383,10 +493,26 @@ __global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams 
 }
 
 template <int NCH>
-cudaError_t launch_rerank_stream(const RerankParams& p, size_t smem, cudaStream_t st) {
+__global__ void __launch_bounds__(RS_THREADS) rerank_stream_kernel(RerankParams p) {
+  rerank_stream_body<NCH, false>(p, MultiClus{});
+}
+
+template <int NCH>
+__global__ void __launch_bounds__(RS_THREADS) rerank_stream_multiclus_kernel(RerankParams p, MultiClus mc) {
+  rerank_stream_body<NCH, true>(p, mc);
+}
+
+template <int NCH>
+cudaError_t launch_rerank_stream(const RerankParams& p, const MultiClus* mc, size_t smem, cudaStream_t st) {
+  const int64_t grid = (int64_t)p.nq * p.S;
+  if (mc) {
+    cudaError_t e = cudaFuncSetAttribute(rerank_stream_multiclus_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    rerank_stream_multiclus_kernel<NCH><<<(unsigned)grid, RS_THREADS, smem, st>>>(p, *mc);
+    return cudaGetLastError();
+  }
   cudaError_t e = cudaFuncSetAttribute(rerank_stream_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  const int64_t grid = (int64_t)p.nq * p.S;
   rerank_stream_kernel<NCH><<<(unsigned)grid, RS_THREADS, smem, st>>>(p);
   return cudaGetLastError();
 }
@@ -555,14 +681,14 @@ extern "C" {
 static int cluster_rerank_impl(mevi_ctx* ctx, const float* Q, int nq, const float* D, int64_t n, int d, int d_layout,
                                const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
                                const int32_t* query_leaves, int L, int k, int64_t id_base, float* scores, int64_t* ids,
-                               int32_t* n_candidates, int64_t max_rows, void* stream);
+                               int32_t* n_candidates, int64_t max_rows, const MultiClus* mc, void* stream);
 
 int mevi_cluster_rerank(mevi_ctx* ctx, const float* Q, int nq, const float* D, int64_t n, int d, int d_layout,
                         const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
                         const int32_t* query_leaves, int L, int k, int64_t id_base, float* scores, int64_t* ids,
                         int32_t* n_candidates, void* stream) {
   return cluster_rerank_impl(ctx, Q, nq, D, n, d, d_layout, leaf_offsets, n_leaves, leaf_docids, query_leaves, L, k, id_base,
-                             scores, ids, n_candidates, 0, stream);
+                             scores, ids, n_candidates, 0, nullptr, stream);
 }
 
 // Same, restricted to the first max_rows candidate rows of every query (leaf-ordered layout only): the exact top-k
@@ -574,13 +700,34 @@ int mevi_cluster_rerank_prefix(mevi_ctx* ctx, const float* Q, int nq, const floa
                                int32_t* n_candidates, void* stream) {
   if (ctx && max_rows <= 0) return mevi_set_error(ctx, MEVI_ERR_INVALID, "max_rows must be positive");
   return cluster_rerank_impl(ctx, Q, nq, D_leaf, n, d, 1, leaf_offsets, n_leaves, leaf_docids, query_leaves, L, k, 0, scores, ids,
-                             n_candidates, max_rows, stream);
+                             n_candidates, max_rows, nullptr, stream);
+}
+
+// --doc_multiclus > 1: one entry per (query, document), its score aggregated over the query's leaves that list it.
+int mevi_cluster_rerank_multiclus(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int64_t n, int d,
+                                  const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
+                                  const int32_t* occ_leaves, int C, const int32_t* query_leaves, int L, int k, int aggr,
+                                  int64_t id_base, float* scores, int64_t* ids, int32_t* n_candidates, void* stream) {
+  MEVI_CHECK_CTX(ctx);
+  MEVI_REQUIRE(ctx, aggr == MEVI_MULTICLUS_ADD || aggr == MEVI_MULTICLUS_MAX, "aggr must be MEVI_MULTICLUS_ADD or _MAX (got %d)", aggr);
+  MEVI_REQUIRE(ctx, C >= 1 && (C == 1 || occ_leaves), "C must be >= 1, with an occurrence table when C > 1");
+  MEVI_REQUIRE(ctx, ((uintptr_t)occ_leaves & 15) == 0, "occ_leaves must be 16-byte aligned");
+  if (C > 16)
+    return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "multi-cluster re-rank: a document is listed under %d leaves (at most 16)", C);
+  MultiClus mc;
+  mc.occ_leaves = occ_leaves;
+  mc.C = C;
+  mc.aggr = aggr;
+  mc.hash_log2 = 1;
+  while ((1 << mc.hash_log2) < 2 * L) ++mc.hash_log2;
+  return cluster_rerank_impl(ctx, Q, nq, D_leaf, n, d, 1, leaf_offsets, n_leaves, leaf_docids, query_leaves, L, k, id_base, scores,
+                             ids, n_candidates, 0, &mc, stream);
 }
 
 static int cluster_rerank_impl(mevi_ctx* ctx, const float* Q, int nq, const float* D, int64_t n, int d, int d_layout,
                                const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
                                const int32_t* query_leaves, int L, int k, int64_t id_base, float* scores, int64_t* ids,
-                               int32_t* n_candidates, int64_t max_rows, void* stream) {
+                               int32_t* n_candidates, int64_t max_rows, const MultiClus* mc, void* stream) {
   MEVI_CHECK_CTX(ctx);
   DeviceGuard g(ctx->device);
   cudaStream_t st = (cudaStream_t)stream;
@@ -616,15 +763,16 @@ static int cluster_rerank_impl(mevi_ctx* ctx, const float* Q, int nq, const floa
     p.out_scores = (float*)(ws + (size_t)nq * S * k * sizeof(int64_t));
   }
   size_t smem = (size_t)cap * 8 + (size_t)(2 * L + 1) * sizeof(int64_t);
+  if (mc) smem += (size_t)(3 * (1 << mc->hash_log2) + L) * sizeof(int32_t) + RS_STAGES * RS_OCC_SLOT;  // leaf table, own-leaf counts, table slices
   cudaError_t e;
   const size_t ring = (size_t)RS_STAGES * RS_ROWS * d * 4;
   if (d_layout == 1 && smem + ring + 256 <= 220 * 1024) {
     smem += ring + 128;
-    if (d <= 128) e = launch_rerank_stream<1>(p, smem, st);
-    else if (d <= 256) e = launch_rerank_stream<2>(p, smem, st);
-    else if (d <= 512) e = launch_rerank_stream<4>(p, smem, st);
-    else if (d <= 768) e = launch_rerank_stream<6>(p, smem, st);
-    else e = launch_rerank_stream<8>(p, smem, st);
+    if (d <= 128) e = launch_rerank_stream<1>(p, mc, smem, st);
+    else if (d <= 256) e = launch_rerank_stream<2>(p, mc, smem, st);
+    else if (d <= 512) e = launch_rerank_stream<4>(p, mc, smem, st);
+    else if (d <= 768) e = launch_rerank_stream<6>(p, mc, smem, st);
+    else e = launch_rerank_stream<8>(p, mc, smem, st);
   } else if (d_layout == 1) {
     return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "leaf-ordered re-rank: ring + top-k buffers exceed shared memory (d=%d k=%d L=%d)", d, k, L);
   } else if (d <= 128) e = launch_rerank<1>(p, smem, st);

@@ -35,6 +35,7 @@ class ClusterIndex:
         # int64 [n] or None: document id of local row i when the rows are not one contiguous id range (a leaf-partitioned
         # shard, dist_utils.partition_rows_by_leaf); results are then doc_ids[row] instead of id_base + row
         self.doc_ids = doc_ids
+        self._occ = None
 
     @property
     def n_leaves(self) -> int:
@@ -102,6 +103,15 @@ class ClusterIndex:
         np.cumsum(lens_s, out=offsets[1:])
         return cls(torch.from_numpy(keys_s).to(dev), torch.from_numpy(offsets).to(dev), torch.from_numpy(docids).to(dev),
                    M, K, id_base)
+
+    def occurrence_table(self):
+        """-> (occ int32 [n, C-1], C), built on the device on first use and kept: C is the largest number of leaves that
+        list one document (`--doc_multiclus`; 1 for a single-cluster index, whose table is empty), and row p of occ
+        holds the CSR leaf indices of the document's other positions, -1 padded (-2 - leaf for an earlier position in
+        the same leaf: a leaf that lists the document twice)."""
+        if self._occ is None:
+            self._occ = _lib.get_context(self.device.index).occurrence_table(self.leaf_offsets, self.leaf_docids)
+        return self._occ
 
     # -- queries --------------------------------------------------------------
     def lookup(self, dec) -> torch.Tensor:
@@ -312,14 +322,30 @@ class ClusterReranker:
             self._grouped = dict(row0=row0, nrows=nrows, leaf_tile0=leaf_tile0, img=img, absmax=absmax, maxnorm=maxnorm)
 
     @torch.no_grad()
-    def rerank(self, query_embedding, dec, topk: int = 100):
+    def rerank(self, query_embedding, dec, topk: int = 100, multiclus_score_aggr: Optional[str] = None):
         """-> (scores [nq,k] fp32 desc, ids [nq,k] int64 (-1 padded), n_candidates [nq] int32), on the device.
         With torch.distributed initialised the documents are sharded: every rank scores the
-        candidates it owns, the per-shard lists are all-gathered and merged on every rank."""
+        candidates it owns, the per-shard lists are all-gathered and merged on every rank.
+
+        `multiclus_score_aggr` in ('add', 'max') is the `--doc_multiclus > 1` top-k (main_models.py:3998-4011, then the
+        sort and `[:save_hard_neg]`) for an index that lists a document under up to C <= 16 leaves.  For a query and a
+        document, c = the number of positions of the query's leaf list whose leaf lists the document (a repeated leaf
+        counts once per position, and a leaf listing the document twice counts twice, like the reference's concatenation)
+        and s = its fp32 score, the same at every
+        position.  The document appears once, scored s ('max') or by the fp32 fold ((0 + s) + s) + ... of c terms
+        ('add', the reference's order; for c <= 2 it equals rerank_all's scatter_add_ bit for bit).  The k best
+        distinct documents by (score desc, id asc), rerank_all's order; n_candidates counts occurrences (cur_ndoc).
+        The streaming kernel keeps only the occurrence at the earliest position of the leaf list and scores it
+        agg(c, s) (last_path = "stream-multiclus").  Row-block shards (`from_cluster_dict(row_range=...)`) keep every
+        occurrence of a document on one rank, so the all-gather + merge stays exact; a leaf-partitioned shard
+        (index.doc_ids set) can hold a document's other leaves on other ranks and raises NotImplementedError.
+        None: the single-cluster path, unchanged."""
         dev = self.D.device
         if not isinstance(query_embedding, torch.Tensor):
             query_embedding = torch.from_numpy(np.ascontiguousarray(query_embedding, dtype=np.float32))
         Q = query_embedding.to(device=dev, dtype=torch.float32).contiguous()
+        if multiclus_score_aggr is not None:
+            return self._rerank_multiclus(Q, dec, topk, multiclus_score_aggr)
         ql = self.index.lookup(dec)
         use_grouped = self._grouped is not None and (
             self.mode == "grouped" or ql.numel() >= self.AUTO_QUERIES_PER_LEAF * max(1, self.index.n_leaves))
@@ -345,6 +371,28 @@ class ClusterReranker:
             scores, ids = self.ctx.topk_merge(s_all.contiguous(), i_all.contiguous())
             torch.distributed.all_reduce(ncand)
         return scores, ids, ncand
+
+
+def _rerank_multiclus(self, Q, dec, topk, aggr):
+    if aggr not in ("add", "max"):
+        raise ValueError("multiclus_score_aggr must be 'add' or 'max' (main_models.py:4002-4009)")
+    if self.index.doc_ids is not None:
+        raise NotImplementedError("multi-cluster re-rank on a leaf-partitioned shard: a document's other leaves can live "
+                                  "on other ranks")
+    if not self.leaf_ordered:
+        raise ValueError("multi-cluster re-rank needs the leaf-ordered layout")
+    idx = self.index
+    occ, n_occ = idx.occurrence_table()
+    scores, ids, ncand = self.ctx.cluster_rerank_multiclus(Q, self.D, idx.leaf_offsets, idx.leaf_docids, occ, n_occ,
+                                                           idx.lookup(dec), topk, aggr, id_base=idx.id_base)
+    self.last_path = "stream-multiclus"
+    if dist_on():
+        scores, ids = self.ctx.topk_merge(all_gather_stack(scores).contiguous(), all_gather_stack(ids).contiguous())
+        torch.distributed.all_reduce(ncand)
+    return scores, ids, ncand
+
+
+ClusterReranker._rerank_multiclus = _rerank_multiclus
 
 
 @torch.no_grad()
