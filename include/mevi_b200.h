@@ -306,6 +306,27 @@ int mevi_rerank_grouped_plan_fill(mevi_ctx* ctx, int round, int32_t* item_tile, 
 int mevi_rerank_grouped_thresholds(mevi_ctx* ctx, int nq, int d, float* tau, int raise, void* stream);
 int mevi_rerank_grouped_finish(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int d, int k, float* scores,
                                int64_t* rows, int32_t* failed_or_null, int* n_failed, void* stream);
+/* The same call on a multi-cluster index (`--doc_multiclus > 1`): the result of mevi_cluster_rerank_multiclus, bit for
+ * bit.  After _begin (tau0 = NULL), _multiclus attaches the index's multi-cluster data to the call:
+ *   query_leaves [nq,L] int32 the query's CSR leaves as given (a repeated leaf included: c counts every position),
+ *   occ_leaves / C from mevi_occurrence_table (NULL when C == 1), tile_leaf [n_tiles] int32 leaf of every image tile,
+ *   aggr MEVI_MULTICLUS_ADD / _MAX.
+ * It writes query_leaves_masked [nq,L] int32 (every later position of a repeated leaf and every empty leaf set to -1:
+ * the list to plan the rounds with, one pair per distinct leaf) and n_candidates [nq] int32 (occurrences, the
+ * reference's cur_ndoc).  The rounds then keep one entry per (query, document), scored by its aggregated approximate
+ * score, against a margin widened for the aggregation (DESIGN §4).  The thresholds of mevi_cluster_rerank_prefix
+ * are not lower bounds here: a query without a usable threshold sample is given tau = +inf (_thresholds, raise != 0)
+ * and re-run by the caller through mevi_cluster_rerank_multiclus.  _finish_multiclus: scores [nq,k] fp32 and
+ * ids [nq,k] int64 = id_base + leaf_docids[row], ordered by (aggregated score desc, id asc), -1 padded; failed / n_failed
+ * as _finish.  query_leaves, leaf_offsets, occ_leaves and tile_leaf must stay valid until _finish_multiclus.
+ * MEVI_ERR_UNSUPPORTED for C > 16 or L > 4096.                                                                      */
+int mevi_rerank_grouped_multiclus(mevi_ctx* ctx, int nq, int d, const int32_t* query_leaves, int L,
+                                  const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* occ_leaves, int C,
+                                  const int32_t* tile_leaf, int aggr, int32_t* query_leaves_masked, int32_t* n_candidates,
+                                  void* stream);
+int mevi_rerank_grouped_finish_multiclus(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int d, int k,
+                                         const int32_t* leaf_docids, int64_t id_base, float* scores, int64_t* ids,
+                                         int32_t* failed_or_null, int* n_failed, void* stream);
 
 /* out[i,:] = D[rows[i],:] for i < m: builds the leaf-ordered copy of the document matrix
  * (rows = the CSR's leaf_docids).  Replaces the per-leaf memmap fancy-index gather of

@@ -56,6 +56,8 @@ SYMBOLS = {
     "mevi_rerank_grouped_plan_fill": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "mevi_rerank_grouped_thresholds": (_i, [_vp, _i, _i, _vp, _i, _vp]),
     "mevi_rerank_grouped_finish": (_i, [_vp, _vp, _i, _vp, _i, _i, _vp, _vp, _vp, C.POINTER(_i), _vp]),
+    "mevi_rerank_grouped_multiclus": (_i, [_vp, _i, _i, _vp, _i, _vp, _i64, _vp, _i, _vp, _i, _vp, _vp, _vp]),
+    "mevi_rerank_grouped_finish_multiclus": (_i, [_vp, _vp, _i, _vp, _i, _i, _vp, _i64, _vp, _vp, _vp, C.POINTER(_i), _vp]),
     "mevi_gather_rows": (_i, [_vp, _vp, _i64, _i, _vp, _i64, _vp, _vp]),
     "mevi_flat_ip_topk": (_i, [_vp, _vp, _i, _vp, _i64, _i, _i, _i64, _i, _vp, _vp, _vp]),
     "mevi_flat_index_create": (_i, [_vp, _vp, _i64, _i, C.POINTER(_vp), _vp]),
@@ -626,6 +628,40 @@ class Context:
             self._check(self.lib.mevi_rerank_grouped_finish(self.handle, _ptr(Q), nq, _ptr(D_leaf), d, int(k), _ptr(scores),
                                                             _ptr(rows), _ptr(failed), C.byref(nf), self._stream()))
         return scores, rows, failed, int(nf.value)
+
+    def rerank_grouped_multiclus(self, Q, query_leaves, leaf_offsets, occ, n_occ, tile_leaf, aggr):
+        """Attach a multi-cluster index to the grouped call begun by rerank_grouped_begin -> (query_leaves with every later
+        position of a repeated leaf set to -1: the list to plan the rounds with, n_candidates int32 [nq])."""
+        import torch
+
+        ql = self._dev(query_leaves, torch.int32, "query_leaves")
+        lo = self._dev(leaf_offsets, torch.int64, "leaf_offsets")
+        tl = self._dev(tile_leaf, torch.int32, "tile_leaf")
+        occ = self._dev(occ, torch.int32, "occ")
+        nq, L = ql.shape
+        masked = torch.empty_like(ql)
+        ncand = torch.empty(nq, dtype=torch.int32, device=ql.device)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mevi_rerank_grouped_multiclus(
+                self.handle, nq, Q.shape[1], _ptr(ql), L, _ptr(lo), lo.numel() - 1, _ptr(occ) if occ.numel() else None,
+                int(n_occ), _ptr(tl), _MULTICLUS_AGGR[aggr], _ptr(masked), _ptr(ncand), self._stream()))
+        return masked, ncand
+
+    def rerank_grouped_finish_multiclus(self, Q, D_leaf, k, leaf_docids, id_base=0):
+        """-> (scores, ids int64 document ids, failed int32 [nq] device mask, n_failed); n_failed == nq: the call is invalid."""
+        import torch
+
+        ld = self._dev(leaf_docids, torch.int32, "leaf_docids")
+        nq, d = Q.shape
+        scores = torch.empty((nq, k), dtype=torch.float32, device=Q.device)
+        ids = torch.empty((nq, k), dtype=torch.int64, device=Q.device)
+        failed = torch.empty(nq, dtype=torch.int32, device=Q.device)
+        nf = C.c_int(nq)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mevi_rerank_grouped_finish_multiclus(self.handle, _ptr(Q), nq, _ptr(D_leaf), d, int(k), _ptr(ld),
+                                                                      int(id_base), _ptr(scores), _ptr(ids), _ptr(failed),
+                                                                      C.byref(nf), self._stream()))
+        return scores, ids, failed, int(nf.value)
 
     def flat_ip_topk(self, Q, D, k, id_base=0, mode="auto"):
         import torch

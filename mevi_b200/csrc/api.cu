@@ -146,6 +146,7 @@ void mevi_ctx_destroy(mevi_ctx* ctx) {
   for (int i = 0; i < 4; ++i)
     if (ctx->aux_event[i]) cudaEventDestroy(ctx->aux_event[i]);
   free(ctx->gr_plan);
+  free(ctx->gr_mc);
   delete ctx;
 }
 

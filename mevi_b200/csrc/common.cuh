@@ -28,6 +28,7 @@ enum WsSlot {
   WS_PQ_PAD,        // PQ encode on the tensor path: block-padded codebook
   WS_FLAT_IMAGE,    // one-shot flat search: fp16 image of the documents (+ its metadata)
   WS_GR_PLAN,       // grouped re-rank: device-side round plan (counts, scans, arrival numbers)
+  WS_GR_MC,         // grouped re-rank of a multi-cluster index: per-query leaf tables, prefilter factors, margins
   WS_NUM
 };
 
@@ -53,6 +54,8 @@ struct mevi_ctx {
   // host-side state of the grouped re-rank's round plan between mevi_rerank_grouped_plan and its _plan_fill calls
   // (rerank_plan.cu owns the layout; malloc'ed, freed with the context)
   void* gr_plan = nullptr;
+  // host-side state of a multi-cluster grouped call between mevi_rerank_grouped_multiclus and its _finish (flat_tensor.cu)
+  void* gr_mc = nullptr;
   int64_t launches = 0;            // kernels launched by this context (reported by mevi_device_info)
 };
 

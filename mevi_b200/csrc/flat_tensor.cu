@@ -20,6 +20,7 @@
 // blocks.  Roofline: tensor pipe (2*nq*N*d FLOP); L2->SM operand traffic is the practical limiter.
 #include <cuda_fp16.h>
 #include <math_constants.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -756,9 +757,57 @@ struct GroupedParams {
   const float* consts; const float* tau; const float* margin;
   int* count; float* cand_score; int32_t* cand_id; int* overflow; int capg;
   int* err_flag;
+  // multi-cluster index (MC instantiation only; see "Multi-cluster indexes" below)
+  const int32_t* occ; int occ_w;  // [rows][occ_w] CSR leaves of the document's other positions (occurrence table), occ_w = C - 1
+  const int32_t* tile_leaf;       // [n_tiles] leaf of every image tile
+  const uint64_t* qtab; int qtab_log2;  // [nq][1 << qtab_log2] per-query leaf tables (mc_probe)
+  const float* mc_cheap;          // [nq] factor applied to a positive threshold for the one-compare prefilter
+  int aggr;                       // MEVI_MULTICLUS_ADD / _MAX
 };
 
-template <int MAXG>
+// ---- Multi-cluster indexes (--doc_multiclus > 1) ----------------------------------------------------------------------
+// A document listed under several leaves has several rows of the leaf-ordered matrix (CSR positions).  For a query q
+// and a document, c = the number of positions of q's leaf list whose leaf lists the document; the kept occurrence is
+// the canonical one of rerank.cu: the earliest position of the list, the first CSR position inside that leaf.  Per query
+// an open-addressed table (1 << qtab_log2 >= 2L slots, rerank.cu's hash) maps a leaf to one 64-bit word: leaf (bits
+// 0-31; 0xFFFFFFFF = empty), its first position in the list (32-47) and its number of positions (48-63).
+__device__ __forceinline__ uint64_t mc_probe(const uint64_t* __restrict__ tab, int log2, int leaf) {
+  const unsigned mask = (1u << log2) - 1u;
+  unsigned h = ((unsigned)leaf * 0x9E3779B1u) >> (32 - log2);
+  for (;;) {  // load factor <= 1/2: an empty slot ends every probe sequence
+    const uint64_t e = __ldg(tab + h);
+    if ((uint32_t)e == (uint32_t)leaf || (uint32_t)e == 0xFFFFFFFFu) return e;
+    h = (h + 1) & mask;
+  }
+}
+
+// c of the occurrence (row of leaf `own`, query with table `tab`), or -1 when the occurrence is not canonical.  `own`
+// sits at its first position in the list (the plan holds one pair per distinct leaf).
+__device__ __forceinline__ int mc_count(const uint64_t* __restrict__ tab, int log2, int own, const int32_t* __restrict__ sib,
+                                        int w) {
+  const uint64_t e = mc_probe(tab, log2, own);
+  const int t = (int)((e >> 32) & 0xFFFFu);
+  int c = (int)(e >> 48);
+  for (int i = 0; i < w; ++i) {
+    const int32_t leaf = __ldg(sib + i);
+    if (leaf == -1) break;              // padding
+    if (leaf <= -2) return -1;          // an earlier CSR position of the same leaf
+    const uint64_t f = mc_probe(tab, log2, leaf);
+    if ((uint32_t)f == 0xFFFFFFFFu) continue;  // a leaf the query did not ask for
+    if ((int)((f >> 32) & 0xFFFFu) < t) return -1;
+    c += (int)(f >> 48);
+  }
+  return c;
+}
+
+// the reference's 'add': zeros, then += s once per position (main_models.py:4004-4007), as in rerank.cu
+__device__ __forceinline__ float mc_fold(float s, int c) {
+  float a = 0.f;
+  for (int i = 0; i < c; ++i) a = __fadd_rn(a, s);
+  return a;
+}
+
+template <int MAXG, bool MC>
 __global__ void __launch_bounds__(GR_THREADS, 1) grouped_gemm_kernel(GroupedParams p) {
   constexpr int STAGES = gr_stages(MAXG), STAGE_BYTES = gr_stage_bytes(MAXG), ACC_COLS = MAXG * GR_TN;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -857,7 +906,11 @@ __global__ void __launch_bounds__(GR_THREADS, 1) grouped_gemm_kernel(GroupedPara
       if (etid < GR_TN * ng) {
         const int q = p.group_qid[grp * GR_TN + etid];
         qid[etid] = q;
-        thr[etid] = q >= 0 ? (p.tau[q] - p.margin[q]) * sdsq : CUDART_INF_F;
+        float t = q >= 0 ? (p.tau[q] - p.margin[q]) * sdsq : CUDART_INF_F;
+        // MC 'add': an aggregated score is at most max(s, c_max s) (rounded up), so a positive threshold is divided
+        // by c_max (mc_cheap < 1 / c_max) and ONE compare per accumulator still decides who goes further
+        if constexpr (MC) if (q >= 0 && t > 0.f) t *= p.mc_cheap[q];
+        thr[etid] = t;
       }
       asm volatile("bar.sync 1, %0;" ::"n"(32 * GR_EPI_WARPS) : "memory");
       if (!ptx::mbar_wait_backoff(&acc_full[buf], ph, 64)) { atomicExch(p.err_flag, 4); ok = false; break; }
@@ -895,6 +948,51 @@ __global__ void __launch_bounds__(GR_THREADS, 1) grouped_gemm_kernel(GroupedPara
 #pragma unroll
           for (int j = 0; j < 32; ++j) mk |= (!(__uint_as_float(acc[j]) < thr[c0 + j]) ? 1u : 0u) << j;
           if (!doc_ok) mk = 0;
+          if constexpr (MC) {
+            // the few pairs that passed: drop non-canonical occurrences, aggregate over the query's WHOLE leaf list, apply
+            // the exact test to the aggregated approximate score and append that score.  One column at a time.
+            const int own = p.tile_leaf[tile];
+            const int32_t* sib = p.occ + (int64_t)doc * p.occ_w;
+            const unsigned tab_sz = 1u << p.qtab_log2;
+            for (unsigned cols = __reduce_or_sync(MEVI_FULL_MASK, mk); cols; cols &= cols - 1) {  // warp-uniform
+              const int j = __ffs(cols) - 1;
+              const int q = qid[c0 + j];
+              bool pass = ((mk >> j) & 1u) && q >= 0;
+              float agg = 0.f;
+              if (pass) {
+                // acc[j] for a run-time j without spilling acc[] to local memory: 5-level select tree
+                uint32_t a16[16], a8[8], a4[4], a2[2];
+#pragma unroll
+                for (int i = 0; i < 16; ++i) a16[i] = (j & 16) ? acc[i + 16] : acc[i];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) a8[i] = (j & 8) ? a16[i + 8] : a16[i];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) a4[i] = (j & 4) ? a8[i + 4] : a8[i];
+#pragma unroll
+                for (int i = 0; i < 2; ++i) a2[i] = (j & 2) ? a4[i + 2] : a4[i];
+                const float s = __uint_as_float((j & 1) ? a2[1] : a2[0]) * inv;
+                const int c = mc_count(p.qtab + (int64_t)q * tab_sz, p.qtab_log2, own, sib, p.occ_w);
+                agg = p.aggr == MEVI_MULTICLUS_ADD ? mc_fold(s, c) : s;
+                pass = c >= 0 && !(agg < p.tau[q] - p.margin[q]);
+              }
+              const unsigned m = __ballot_sync(MEVI_FULL_MASK, pass);
+              if (m) {
+                int b0 = 0;
+                if (lane == 0) b0 = atomicAdd(&p.count[q], __popc(m));
+                b0 = __shfl_sync(MEVI_FULL_MASK, b0, 0);
+                if (pass) {
+                  const int slot = b0 + __popc(m & ((1u << lane) - 1u));
+                  if (slot < p.capg) {
+                    p.cand_score[(int64_t)q * p.capg + slot] = agg;
+                    p.cand_id[(int64_t)q * p.capg + slot] = doc;
+                  } else {
+                    p.overflow[q] = 1;
+                  }
+                }
+              }
+            }
+            continue;
+          }
           unsigned mym = 0;  // lane j: documents (lanes) passing column j
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
@@ -1004,13 +1102,18 @@ __global__ void __launch_bounds__(256) gr_group_image_kernel(const __half* __res
   }
 }
 
-template <int MAXG>
+template <int MAXG, bool MC>
 int gr_launch(mevi_ctx* ctx, const GroupedParams& p, int grid, cudaStream_t st) {
   const size_t smem = (size_t)gr_stages(MAXG) * gr_stage_bytes(MAXG) + 2 * MAXG * GR_TN * 8 +
                       (2 * gr_stages(MAXG) + 4) * 8 + 16 + 1024;
-  MEVI_CUDA(ctx, cudaFuncSetAttribute(grouped_gemm_kernel<MAXG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  grouped_gemm_kernel<MAXG><<<grid, GR_THREADS, smem, st>>>(p);
+  MEVI_CUDA(ctx, cudaFuncSetAttribute(grouped_gemm_kernel<MAXG, MC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  grouped_gemm_kernel<MAXG, MC><<<grid, GR_THREADS, smem, st>>>(p);
   return MEVI_OK;
+}
+
+template <bool MC>
+int gr_launch_maxg(mevi_ctx* ctx, const GroupedParams& p, int maxg, int grid, cudaStream_t st) {
+  return maxg == 1 ? gr_launch<1, MC>(ctx, p, grid, st) : (maxg == 2 ? gr_launch<2, MC>(ctx, p, grid, st) : gr_launch<4, MC>(ctx, p, grid, st));
 }
 
 __global__ void gr_set_u32_kernel(unsigned* p, unsigned v) { *p = v; }
@@ -1079,6 +1182,167 @@ bool gr_state(mevi_ctx* ctx, int nq, int d, GrState* s) {
   return true;
 }
 
+// ---- multi-cluster call state (mevi_rerank_grouped_multiclus .. _finish_multiclus) ----
+struct GrMcHost {  // plain data: lives in mevi_ctx::gr_mc
+  int valid, nq, qtab_log2, C, aggr;
+  const int32_t* occ; const int32_t* tile_leaf; const int64_t* leaf_offsets; int64_t n_leaves;
+};
+struct GrMcState { uint64_t* qtab; float* cheap; float* m_mc; };
+
+bool gr_mc_state(mevi_ctx* ctx, int nq, int log2, GrMcState* s) {
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
+  const size_t o_tab = take((size_t)nq * (8u << log2)), o_cheap = take((size_t)nq * 4), o_m = take((size_t)nq * 4);
+  char* ws = (char*)mevi_ws(ctx, WS_GR_MC, off);
+  if (!ws) return false;
+  s->qtab = (uint64_t*)(ws + o_tab); s->cheap = (float*)(ws + o_cheap); s->m_mc = (float*)(ws + o_m);
+  return true;
+}
+
+// the attached multi-cluster state of the current call, or nullptr (a single-cluster call)
+const GrMcHost* gr_mc_attached(mevi_ctx* ctx, int nq) {
+  const GrMcHost* h = (const GrMcHost*)ctx->gr_mc;
+  return h && h->valid && h->nq == nq ? h : nullptr;
+}
+
+// One CTA per query: its leaf table (from the UNMASKED list: c counts every position), n_candidates (every position, like
+// the streaming kernel), the list with every later position of a repeated leaf set to -1 (one plan pair per distinct leaf),
+// and from c_max = C x the largest repetition of a leaf (an upper bound of c):
+//   m_mc = c_max margin + c_max (c_max - 1) 2^-24 (4.05 |q| dmax + 1.01 margin),  x (1 + 2^-13) for its own fp32 evaluation
+//   cheap = 1 / (c_max (1 + (c_max + 4) 2^-21))
+// ('max': m_mc = margin, cheap = 1).  DESIGN §4 derives both.
+__global__ void __launch_bounds__(256) gr_mc_table_kernel(const int32_t* __restrict__ ql, int L, const int64_t* __restrict__ off,
+                                                          int64_t n_leaves, int C, int aggr, int log2, const float* __restrict__ margin,
+                                                          const float* __restrict__ qnorm, const unsigned* __restrict__ dmax_bits,
+                                                          uint64_t* __restrict__ qtab, float* __restrict__ cheap,
+                                                          float* __restrict__ m_mc, int32_t* __restrict__ ql_masked,
+                                                          int32_t* __restrict__ ncand) {
+  extern __shared__ int32_t s_tab[];  // key | first position | number of positions, [1 << log2] each
+  const int H = 1 << log2;
+  int32_t* s_key = s_tab;
+  int32_t* s_first = s_tab + H;
+  int32_t* s_mult = s_tab + 2 * H;
+  __shared__ long long s_tot[8];
+  __shared__ int s_rep[8];
+  const int q = blockIdx.x, tid = threadIdx.x;
+  for (int i = tid; i < H; i += blockDim.x) { s_key[i] = -1; s_first[i] = 0x7fffffff; s_mult[i] = 0; }
+  __syncthreads();
+  long long tot = 0;
+  for (int t = tid; t < L; t += blockDim.x) {
+    const int leaf = ql[(int64_t)q * L + t];
+    if (leaf < 0 || leaf >= n_leaves) continue;
+    const int64_t sz = off[leaf + 1] - off[leaf];
+    tot += sz;
+    if (sz == 0) continue;  // no document: never scored, never a sibling
+    const unsigned mask = (unsigned)H - 1u;
+    unsigned h = ((unsigned)leaf * 0x9E3779B1u) >> (32 - log2);
+    for (;;) {
+      const int prev = atomicCAS(&s_key[h], -1, leaf);
+      if (prev < 0 || prev == leaf) break;
+      h = (h + 1) & mask;
+    }
+    atomicMin(&s_first[h], t);
+    atomicAdd(&s_mult[h], 1);
+  }
+  __syncthreads();
+  int rep = 0;
+  for (int t = tid; t < L; t += blockDim.x) {
+    const int leaf = ql[(int64_t)q * L + t];
+    int keep = -1;
+    if (leaf >= 0 && leaf < n_leaves && off[leaf + 1] > off[leaf]) {
+      unsigned h = ((unsigned)leaf * 0x9E3779B1u) >> (32 - log2);
+      while (s_key[h] != leaf) h = (h + 1) & ((unsigned)H - 1u);
+      if (s_first[h] == t) keep = leaf;
+    }
+    ql_masked[(int64_t)q * L + t] = keep;
+  }
+  for (int i = tid; i < H; i += blockDim.x) {
+    const int k = s_key[i];
+    qtab[(int64_t)q * H + i] = k < 0 ? ~0ull : ((uint64_t)(uint32_t)k | ((uint64_t)s_first[i] << 32) | ((uint64_t)s_mult[i] << 48));
+    rep = max(rep, s_mult[i]);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    tot += __shfl_xor_sync(MEVI_FULL_MASK, tot, o);
+    rep = max(rep, __shfl_xor_sync(MEVI_FULL_MASK, rep, o));
+  }
+  if ((tid & 31) == 0) { s_tot[tid >> 5] = tot; s_rep[tid >> 5] = rep; }
+  __syncthreads();
+  if (tid == 0) {
+    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) { tot += s_tot[w]; rep = max(rep, s_rep[w]); }
+    ncand[q] = (int32_t)(tot > 0x7FFFFFFFll ? 0x7FFFFFFFll : tot);
+    const float cm = (float)max(C * rep, 1), mq = margin[q];
+    if (aggr == MEVI_MULTICLUS_ADD) {
+      const float B = qnorm[q] * __uint_as_float(*dmax_bits);
+      m_mc[q] = (cm * mq + cm * (cm - 1.f) * 5.9604645e-8f * (4.05f * B + 1.01f * mq)) * 1.0001221f;
+      cheap[q] = 1.f / (cm * (1.f + (cm + 4.f) * 4.7683716e-7f));
+    } else {
+      m_mc[q] = mq;
+      cheap[q] = 1.f;
+    }
+  }
+}
+
+// flat_rescore_kernel for a multi-cluster call: the same exact re-score (the dense scorer's summation order, as the
+// streaming kernel), then c from the query's leaf table and the fold; sorted by (aggregated score desc, DOCUMENT id asc):
+// leaf order is not document order when documents sit under several leaves.  ids = id_base + leaf_docids[row].
+__global__ void __launch_bounds__(256) gr_mc_rescore_kernel(const float* __restrict__ Q, const float* __restrict__ D, int d,
+                                                            const int* __restrict__ count, const int32_t* __restrict__ cand_id,
+                                                            const float* __restrict__ cand_score, const float* __restrict__ tau,
+                                                            const float* __restrict__ margin, int capg, int k, int keep_pow2,
+                                                            const int64_t* __restrict__ off, int64_t n_leaves,
+                                                            const int32_t* __restrict__ occ, int occ_w,
+                                                            const uint64_t* __restrict__ qtab, int log2, int aggr,
+                                                            const int32_t* __restrict__ leaf_docids, int64_t id_base,
+                                                            float* __restrict__ scores, int64_t* __restrict__ ids) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float* s_score = reinterpret_cast<float*>(smem_raw);
+  int32_t* s_id = reinterpret_cast<int32_t*>(s_score + keep_pow2);
+  const int q = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int cnt = count[q];
+  if (cnt > keep_pow2) cnt = keep_pow2;
+  for (int i = threadIdx.x; i < keep_pow2; i += blockDim.x) {
+    s_score[i] = -CUDART_INF_F;
+    s_id[i] = 0x7fffffff;
+  }
+  __syncthreads();
+  const float window = tau[q] - margin[q];
+  for (int i = warp; i < cnt; i += 8) {
+    if (cand_score[(int64_t)q * capg + i] < window) continue;
+    const int32_t row = cand_id[(int64_t)q * capg + i];
+    float acc = 0.f;
+    for (int c4 = lane * 4; c4 < d; c4 += 128) {  // same summation pattern as the dense scorer
+      const float4 a = ldg_f4(Q + (int64_t)q * d + c4);
+      const float4 b = ld_stream_f4(D + (int64_t)row * d + c4);
+      acc = fmaf(a.x, b.x, acc);
+      acc = fmaf(a.y, b.y, acc);
+      acc = fmaf(a.z, b.z, acc);
+      acc = fmaf(a.w, b.w, acc);
+    }
+    acc = warp_sum(acc);
+    if (lane == 0) {
+      if (aggr == MEVI_MULTICLUS_ADD) {
+        int64_t lo = 0, hi = n_leaves;  // leaf of the row: last leaf whose first row is <= row
+        while (hi - lo > 1) {
+          const int64_t mid = (lo + hi) >> 1;
+          if (off[mid] <= row) lo = mid; else hi = mid;
+        }
+        // every kept occurrence is canonical, so c >= 1
+        acc = mc_fold(acc, mc_count(qtab + ((int64_t)q << log2), log2, (int)lo, occ + (int64_t)row * occ_w, occ_w));
+      }
+      s_score[i] = acc;
+      s_id[i] = leaf_docids[row];
+    }
+  }
+  __syncthreads();
+  block_bitonic_sort<int32_t>(s_score, s_id, keep_pow2);
+  for (int i = threadIdx.x; i < k; i += blockDim.x) {
+    const bool ok = i < cnt && s_id[i] != 0x7fffffff;
+    scores[(int64_t)q * k + i] = ok ? s_score[i] : -CUDART_INF_F;
+    ids[(int64_t)q * k + i] = ok ? id_base + (int64_t)s_id[i] : -1;
+  }
+}
+
 }  // namespace
 
 // fp16 image of the leaf-ordered matrix, tiles of 128 rows that never straddle a leaf.
@@ -1129,6 +1393,7 @@ extern "C" int mevi_rerank_grouped_begin(mevi_ctx* ctx, const float* Q, int nq, 
   MEVI_REQUIRE(ctx, Q && nq > 0 && d_absmax >= 0.f, "bad argument");
   GrState s;
   if (!gr_state(ctx, nq, d, &s)) return MEVI_ERR_NOMEM;
+  if (ctx->gr_mc) ((GrMcHost*)ctx->gr_mc)->valid = 0;  // a new call: single-cluster unless _multiclus attaches its state
   gr_init_kernel<<<(nq + 255) / 256, 256, 0, st>>>(s.tau, tau0, s.count, s.flags, s.ovq, nq);
   gr_set_u32_kernel<<<1, 1, 0, st>>>(s.absmax + 0, gr_f32_bits(d_absmax));
   gr_set_u32_kernel<<<1, 1, 0, st>>>(s.absmax + 1, 0u);
@@ -1173,13 +1438,20 @@ extern "C" int mevi_rerank_grouped_round(mevi_ctx* ctx, const float* Q, int nq, 
   p.tile_row0 = tile_row0; p.tile_nrows = tile_nrows; p.group_qid = group_qid; p.group_ncols = group_ncols; p.nchunks = nchunks;
   p.consts = s.consts; p.tau = s.tau; p.margin = s.margin; p.count = s.count; p.cand_score = s.cand_score;
   p.cand_id = s.cand_id; p.overflow = s.ovq; p.capg = GR_CAPG; p.err_flag = s.flags + 1;
+  p.occ = nullptr; p.occ_w = 0; p.tile_leaf = nullptr; p.qtab = nullptr; p.qtab_log2 = 1; p.mc_cheap = nullptr; p.aggr = 0;
+  const GrMcHost* mc = gr_mc_attached(ctx, nq);
+  if (mc) {  // multi-cluster call: the MC epilogue, and the aggregated margin for it and for the compaction
+    GrMcState ms;
+    if (!gr_mc_state(ctx, nq, mc->qtab_log2, &ms)) return MEVI_ERR_NOMEM;
+    p.margin = ms.m_mc; p.occ = mc->occ; p.occ_w = mc->C - 1; p.tile_leaf = mc->tile_leaf; p.qtab = ms.qtab;
+    p.qtab_log2 = mc->qtab_log2; p.mc_cheap = ms.cheap; p.aggr = mc->aggr;
+  }
   const int grid = (int)(n_items < ctx->sm_count ? n_items : ctx->sm_count);
   const int maxg = max_groups_per_item <= 1 ? 1 : (max_groups_per_item == 2 ? 2 : 4);
-  if (int rc = maxg == 1 ? gr_launch<1>(ctx, p, grid, st) : (maxg == 2 ? gr_launch<2>(ctx, p, grid, st) : gr_launch<4>(ctx, p, grid, st)))
-    return rc;
+  if (int rc = mc ? gr_launch_maxg<true>(ctx, p, maxg, grid, st) : gr_launch_maxg<false>(ctx, p, maxg, grid, st)) return rc;
   const size_t smem_compact = (size_t)GR_CAPG * 8;
   MEVI_CUDA(ctx, cudaFuncSetAttribute(flat_tensor_compact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_compact));
-  flat_tensor_compact_kernel<<<nq, 256, smem_compact, st>>>(s.tau, s.margin, s.count, s.cand_score, s.cand_id, s.ovq, GR_CAPG, k,
+  flat_tensor_compact_kernel<<<nq, 256, smem_compact, st>>>(s.tau, p.margin, s.count, s.cand_score, s.cand_id, s.ovq, GR_CAPG, k,
                                                             FT_KEEP, 1);
   MEVI_CUDA(ctx, cudaGetLastError());
   MEVI_COUNT_LAUNCH(ctx, 4);
@@ -1216,12 +1488,11 @@ extern "C" int mevi_rerank_grouped_thresholds(mevi_ctx* ctx, int nq, int d, floa
 // (-1 padded), *n_failed = number of queries whose guarantee could not be established (candidate buffer or margin window
 // overflow: near-duplicate documents, one huge leaf) and failed_or_null [nq] (device, int32) marks them: the caller
 // re-runs just those through mevi_cluster_rerank.
-extern "C" int mevi_rerank_grouped_finish(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int d, int k,
-                                          float* scores, int64_t* rows, int32_t* failed_or_null, int* n_failed, void* stream) {
-  MEVI_CHECK_CTX(ctx);
-  DeviceGuard g(ctx->device);
-  cudaStream_t st = (cudaStream_t)stream;
-  MEVI_REQUIRE(ctx, Q && D_leaf && scores && rows && n_failed, "NULL argument");
+namespace {
+// _finish and _finish_multiclus (mc != nullptr: rows -> document ids, see gr_mc_rescore_kernel)
+int gr_finish(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int d, int k, const GrMcHost* mc,
+              const int32_t* leaf_docids, int64_t id_base, float* scores, int64_t* rows, int32_t* failed_or_null, int* n_failed,
+              cudaStream_t st) {
   *n_failed = nq;
   GrState s;
   if (!gr_state(ctx, nq, d, &s)) return MEVI_ERR_NOMEM;
@@ -1235,12 +1506,79 @@ extern "C" int mevi_rerank_grouped_finish(mevi_ctx* ctx, const float* Q, int nq,
   if (h_flags[1]) return mevi_set_error(ctx, MEVI_ERR_CUDA, "grouped re-rank pipeline time-out (code %d)", h_flags[1]);
   if (h_flags[2]) return MEVI_OK;  // clamped query image: nothing of this call carries the guarantee
   const size_t smem_rescore = (size_t)FT_KEEP * 8;
-  flat_rescore_kernel<<<nq, 256, smem_rescore, st>>>(Q, D_leaf, d, s.count, s.cand_id, s.cand_score, s.tau, s.margin, GR_CAPG, k,
-                                                     FT_KEEP, 0, scores, rows);
+  if (mc) {
+    GrMcState ms;
+    if (!gr_mc_state(ctx, nq, mc->qtab_log2, &ms)) return MEVI_ERR_NOMEM;
+    gr_mc_rescore_kernel<<<nq, 256, smem_rescore, st>>>(Q, D_leaf, d, s.count, s.cand_id, s.cand_score, s.tau, ms.m_mc, GR_CAPG, k,
+                                                        FT_KEEP, mc->leaf_offsets, mc->n_leaves, mc->occ, mc->C - 1, ms.qtab,
+                                                        mc->qtab_log2, mc->aggr, leaf_docids, id_base, scores, rows);
+  } else {
+    flat_rescore_kernel<<<nq, 256, smem_rescore, st>>>(Q, D_leaf, d, s.count, s.cand_id, s.cand_score, s.tau, s.margin, GR_CAPG, k,
+                                                       FT_KEEP, 0, scores, rows);
+  }
   MEVI_CUDA(ctx, cudaGetLastError());
   MEVI_COUNT_LAUNCH(ctx, 1);
   *n_failed = h_flags[3];
   return MEVI_OK;
+}
+}  // namespace
+
+extern "C" int mevi_rerank_grouped_finish(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int d, int k,
+                                          float* scores, int64_t* rows, int32_t* failed_or_null, int* n_failed, void* stream) {
+  MEVI_CHECK_CTX(ctx);
+  DeviceGuard g(ctx->device);
+  MEVI_REQUIRE(ctx, Q && D_leaf && scores && rows && n_failed, "NULL argument");
+  return gr_finish(ctx, Q, nq, D_leaf, d, k, nullptr, nullptr, 0, scores, rows, failed_or_null, n_failed, (cudaStream_t)stream);
+}
+
+// Multi-cluster index (--doc_multiclus > 1): attach the call's multi-cluster state after _begin; _round then runs the MC
+// epilogue and _finish_multiclus ends the call.
+extern "C" int mevi_rerank_grouped_multiclus(mevi_ctx* ctx, int nq, int d, const int32_t* query_leaves, int L,
+                                             const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* occ_leaves, int C,
+                                             const int32_t* tile_leaf, int aggr, int32_t* query_leaves_masked,
+                                             int32_t* n_candidates, void* stream) {
+  MEVI_CHECK_CTX(ctx);
+  DeviceGuard g(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  MEVI_REQUIRE(ctx, query_leaves && leaf_offsets && tile_leaf && query_leaves_masked && n_candidates, "NULL argument");
+  MEVI_REQUIRE(ctx, nq > 0 && d > 0 && L > 0 && n_leaves > 0, "bad extents");
+  MEVI_REQUIRE(ctx, aggr == MEVI_MULTICLUS_ADD || aggr == MEVI_MULTICLUS_MAX, "aggr must be MEVI_MULTICLUS_ADD or _MAX (got %d)", aggr);
+  MEVI_REQUIRE(ctx, C >= 1 && (C == 1 || occ_leaves), "C must be >= 1, with an occurrence table when C > 1");
+  if (C > 16 || L > 4096)
+    return mevi_set_error(ctx, MEVI_ERR_UNSUPPORTED, "grouped multi-cluster re-rank: C = %d (at most 16), L = %d (at most 4096)", C, L);
+  GrState s;
+  if (!gr_state(ctx, nq, d, &s)) return MEVI_ERR_NOMEM;
+  int log2 = 1;
+  while ((1 << log2) < 2 * L) ++log2;
+  GrMcState ms;
+  if (!gr_mc_state(ctx, nq, log2, &ms)) return MEVI_ERR_NOMEM;
+  if (!ctx->gr_mc) ctx->gr_mc = calloc(1, sizeof(GrMcHost));
+  if (!ctx->gr_mc) return mevi_set_error(ctx, MEVI_ERR_NOMEM, "grouped multi-cluster re-rank: host state");
+  const size_t smem = (size_t)12 << log2;
+  MEVI_CUDA(ctx, cudaFuncSetAttribute(gr_mc_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  gr_mc_table_kernel<<<nq, 256, smem, st>>>(query_leaves, L, leaf_offsets, n_leaves, C, aggr, log2, s.margin, s.qnorm, s.absmax + 2,
+                                            ms.qtab, ms.cheap, ms.m_mc, query_leaves_masked, n_candidates);
+  MEVI_CUDA(ctx, cudaGetLastError());
+  MEVI_COUNT_LAUNCH(ctx, 1);
+  GrMcHost& h = *(GrMcHost*)ctx->gr_mc;
+  h.nq = nq; h.qtab_log2 = log2; h.C = C; h.aggr = aggr; h.occ = C > 1 ? occ_leaves : nullptr; h.tile_leaf = tile_leaf;
+  h.leaf_offsets = leaf_offsets; h.n_leaves = n_leaves;
+  h.valid = 1;
+  return MEVI_OK;
+}
+
+extern "C" int mevi_rerank_grouped_finish_multiclus(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int d, int k,
+                                                    const int32_t* leaf_docids, int64_t id_base, float* scores, int64_t* ids,
+                                                    int32_t* failed_or_null, int* n_failed, void* stream) {
+  MEVI_CHECK_CTX(ctx);
+  DeviceGuard g(ctx->device);
+  MEVI_REQUIRE(ctx, Q && D_leaf && leaf_docids && scores && ids && n_failed, "NULL argument");
+  const GrMcHost* mc = gr_mc_attached(ctx, nq);
+  MEVI_REQUIRE(ctx, mc, "no multi-cluster state: call mevi_rerank_grouped_multiclus after _begin");
+  const int rc = gr_finish(ctx, Q, nq, D_leaf, d, k, mc, leaf_docids, id_base, scores, ids, failed_or_null, n_failed,
+                           (cudaStream_t)stream);
+  ((GrMcHost*)ctx->gr_mc)->valid = 0;
+  return rc;
 }
 
 

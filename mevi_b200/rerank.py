@@ -383,9 +383,16 @@ def _rerank_multiclus(self, Q, dec, topk, aggr):
         raise ValueError("multi-cluster re-rank needs the leaf-ordered layout")
     idx = self.index
     occ, n_occ = idx.occurrence_table()
-    scores, ids, ncand = self.ctx.cluster_rerank_multiclus(Q, self.D, idx.leaf_offsets, idx.leaf_docids, occ, n_occ,
-                                                           idx.lookup(dec), topk, aggr, id_base=idx.id_base)
-    self.last_path = "stream-multiclus"
+    ql = idx.lookup(dec)
+    # the grouped path under the single-cluster call's conditions (mode, pairs per leaf; _rerank_grouped: image, topk)
+    use_grouped = self._grouped is not None and n_occ <= 16 and ql.shape[1] <= 4096 and (
+        self.mode == "grouped" or ql.numel() >= self.AUTO_QUERIES_PER_LEAF * max(1, idx.n_leaves))
+    out = self._rerank_grouped(Q, ql, topk, multiclus=(occ, n_occ, aggr)) if use_grouped else None
+    if out is None:
+        out = self.ctx.cluster_rerank_multiclus(Q, self.D, idx.leaf_offsets, idx.leaf_docids, occ, n_occ, ql, topk, aggr,
+                                                id_base=idx.id_base)
+        self.last_path = "stream-multiclus"
+    scores, ids, ncand = out
     if dist_on():
         scores, ids = self.ctx.topk_merge(all_gather_stack(scores).contiguous(), all_gather_stack(ids).contiguous())
         torch.distributed.all_reduce(ncand)
@@ -543,16 +550,29 @@ def plan_grouped_tile_rounds(leaf_tile0: torch.Tensor, ql: torch.Tensor, boot_le
     return out
 
 
-def _rerank_grouped(self, Q, ql, topk):
+def _rerank_grouped(self, Q, ql, topk, multiclus=None):
     """Leaf-grouped tensor-core path; None when it does not apply or could not establish its guarantee for the call.
     Queries whose own guarantee fails (candidate buffer or margin-window overflow: near-duplicate documents, one huge
-    leaf) are re-run through the streaming kernel and patched in; the answer is always the exact one."""
+    leaf) are re-run through the streaming kernel and patched in; the answer is always the exact one.
+    multiclus = (occ, C, aggr): the multi-cluster top-k of _rerank_multiclus (one entry per document, aggregated
+    scores; DESIGN §4), bit-equal to mevi_cluster_rerank_multiclus, which re-runs the failed and the weak queries."""
     g = self._grouped
     if g["absmax"] < 0 or topk > 256 or Q.shape[0] == 0:
         return None
     ctx, idx = self.ctx, self.index
     off = idx.leaf_offsets
     boot = (self.BOOT_LEAVES,) if isinstance(self.BOOT_LEAVES, int) else tuple(self.BOOT_LEAVES)
+    ql_all = ql
+    if multiclus is not None:
+        # the multi-cluster state hangs off the call's state (margins, norms): _begin first.  The plan sees one pair per
+        # distinct leaf; c and n_candidates count every position of the unmasked list.
+        if "tile_leaf" not in g:
+            lt0 = g["leaf_tile0"]
+            g["tile_leaf"] = torch.repeat_interleave(torch.arange(lt0.numel() - 1, device=lt0.device, dtype=torch.int32),
+                                                     lt0[1:] - lt0[:-1]).contiguous()
+        ctx.rerank_grouped_begin(Q, g["absmax"], g["maxnorm"], None)
+        ql, ncand_mc = ctx.rerank_grouped_multiclus(Q, ql_all.contiguous(), off, multiclus[0], multiclus[1], g["tile_leaf"],
+                                                    multiclus[2])
     # thresholds bootstrap themselves: the first round (first tiles of the leading leaves of every query) runs without
     # thresholds and appends every score; its compaction yields each query's first k-th best score, the sample rounds
     # that follow tighten it.  A query whose sample is too small for its candidate count (its k-th best would let more
@@ -577,18 +597,27 @@ def _rerank_grouped(self, Q, ql, topk):
         need = torch.clamp(ncand * topk // self.PASS_BUDGET, min=2 * topk).clamp(max=self.BOOTSTRAP_MIN)
         weak = torch.nonzero((ncand > self.PASS_BUDGET) & (boot_rows < need) & (ncand > boot_rows)).squeeze(1)
         ncand = ncand.clamp(max=0x7FFFFFFF).to(torch.int32)
-    tau0 = None
-    if weak.numel():
-        s0, _, _ = ctx.cluster_rerank_prefix(Q[weak].contiguous(), self.D, off, idx.leaf_docids, ql[weak].contiguous(), topk,
-                                             self.BOOTSTRAP_MIN)
-        tau0 = torch.full((Q.shape[0],), float("-inf"), dtype=torch.float32, device=Q.device)
-        tau0[weak] = s0[:, topk - 1]
     self.last_weak_queries = int(weak.numel())
-    ctx.rerank_grouped_begin(Q, g["absmax"], g["maxnorm"], tau0)
+    if multiclus is not None:
+        # the prefix's k-th best OCCURRENCE score is no lower bound of the aggregated k-th best: a weak query gets
+        # tau = +inf (the rounds append nothing for it) and is re-run whole through the streaming kernel
+        ncand = ncand_mc
+        if weak.numel():
+            tau = torch.full((Q.shape[0],), float("-inf"), dtype=torch.float32, device=Q.device)
+            tau[weak] = float("inf")
+            ctx.rerank_grouped_thresholds(Q, tau)
+    else:
+        tau0 = None
+        if weak.numel():
+            s0, _, _ = ctx.cluster_rerank_prefix(Q[weak].contiguous(), self.D, off, idx.leaf_docids, ql[weak].contiguous(), topk,
+                                                 self.BOOTSTRAP_MIN)
+            tau0 = torch.full((Q.shape[0],), float("-inf"), dtype=torch.float32, device=Q.device)
+            tau0[weak] = s0[:, topk - 1]
+        ctx.rerank_grouped_begin(Q, g["absmax"], g["maxnorm"], tau0)
     def share_thresholds():
         # documents sharded over ranks: the largest of the ranks' k-th best scores bounds the global k-th best from below,
         # so after an all-reduce(MAX) of [nq] floats every rank filters the next round - and re-scores - against it
-        if getattr(self, "_share_now", False):
+        if multiclus is None and getattr(self, "_share_now", False):
             tau = ctx.rerank_grouped_thresholds(Q)
             torch.distributed.all_reduce(tau, op=torch.distributed.ReduceOp.MAX)
             ctx.rerank_grouped_thresholds(Q, tau)
@@ -609,8 +638,24 @@ def _rerank_grouped(self, Q, ql, topk):
                 ctx.rerank_grouped_round(Q, g["img"], g["row0"], g["nrows"], item_tile, item_group, group_qid, topk, maxg)
             if self.PLAN == "tiles":  # (the prefix plan's number of rounds can differ between ranks)
                 share_thresholds()
-    scores, rows, failed, n_failed = ctx.rerank_grouped_finish(Q, self.D, topk)
     nq = Q.shape[0]
+    if multiclus is not None:
+        scores, ids, failed, n_failed = ctx.rerank_grouped_finish_multiclus(Q, self.D, topk, idx.leaf_docids, idx.id_base)
+        self.last_failed_queries = n_failed
+        if n_failed >= nq or n_failed > max(16, nq // 4):
+            return None
+        self.last_path = "grouped-multiclus"
+        if n_failed > 0 or weak.numel():
+            rerun = failed != 0
+            rerun[weak] = True
+            bad = torch.nonzero(rerun).squeeze(1)
+            s2, i2, _ = ctx.cluster_rerank_multiclus(Q[bad].contiguous(), self.D, off, idx.leaf_docids, multiclus[0], multiclus[1],
+                                                     ql_all[bad].contiguous(), topk, multiclus[2], id_base=idx.id_base)
+            scores[bad] = s2
+            ids[bad] = i2
+            self.last_path = "grouped-multiclus+stream"
+        return scores, ids, ncand
+    scores, rows, failed, n_failed = ctx.rerank_grouped_finish(Q, self.D, topk)
     self.last_failed_queries = n_failed
     if n_failed >= nq or n_failed > max(16, nq // 4):
         return None

@@ -6,7 +6,9 @@ warm-up calls of each:
   (a) rerank(topk=100, multiclus_score_aggr=aggr)            the streaming kernel with the occurrence table
   (b) rerank_all(multiclus_score_aggr=aggr) + truncation     every candidate, aggregated and sorted, then the first 100
   (c) rerank(topk=100) on the single-cluster index            the same corpus, each document under one leaf
-(a) is checked against (b).  The working set (27 GB and 54 GB leaf-ordered matrices) is far larger than L2.
+  (d) (a) on the leaf-grouped tensor-core path (mode="grouped", the same leaf-ordered matrix plus its fp16 tile image)
+(a) is checked against (b), and (d) against (a) bit for bit (ids, fp32 scores, n_candidates); the failed and weak query
+counts of (d) are reported.  The working set (27 GB and 54 GB leaf-ordered matrices) is far larger than L2.
 Prints one JSON line.  Usage: python tools/multiclus_rerank_time.py [--reps 5] [--queries 6980]"""
 import argparse
 import json
@@ -103,6 +105,7 @@ def main():
     rr_sc = ClusterReranker(None, idx_sc, mode="stream", D_leaf=ctx.gather_rows(X, idx_sc.leaf_docids))
     del X
     torch.cuda.empty_cache()
+    rr_mcg = ClusterReranker(None, idx_mc, mode="grouped", D_leaf=rr_mc.D)  # no third copy: only the fp16 image is added
 
     def truncated_all(aggr):
         off, ids, scores = rr_mc.rerank_all(Q, dec, multiclus_score_aggr=aggr)
@@ -129,6 +132,13 @@ def main():
         res[f"b_{aggr}_ms"] = t_b
         res[f"a_{aggr}_mean_candidates"] = float(n_a.float().mean())
         res[f"a_equals_b_{aggr}"] = bool(torch.equal(s_a, s_b) and torch.equal(i_a, i_b))
+        (s_d, i_d, n_d), t_d = timed(lambda: rr_mcg.rerank(Q, dec, topk=topk, multiclus_score_aggr=aggr), args.reps)
+        res[f"d_{aggr}_ms"] = t_d
+        res[f"d_{aggr}_path"] = rr_mcg.last_path
+        res[f"d_{aggr}_failed_queries"] = rr_mcg.last_failed_queries
+        res[f"d_{aggr}_weak_queries"] = rr_mcg.last_weak_queries
+        res[f"d_equals_a_{aggr}"] = bool(torch.equal(i_d, i_a) and torch.equal(s_d.view(torch.int32), s_a.view(torch.int32))
+                                         and torch.equal(n_d, n_a))
     print(json.dumps(res))
 
 
