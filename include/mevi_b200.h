@@ -357,6 +357,22 @@ void mevi_flat_index_destroy(mevi_ctx* ctx, mevi_flat_index* index);
 int mevi_topk_merge(mevi_ctx* ctx, const float* scores_in, const int64_t* ids_in, int S, int nq, int k,
                     float* scores, int64_t* ids, void* stream);
 
+/* Merge S per-shard CSRs of rerank_all (after an all-gather) into the whole corpus's: per query, S runs each sorted by
+ * (score desc, id asc) -> one run in the same order.  -0.0 and +0.0 compare equal, as the device torch.sort orders
+ * them (rerank_all's sort); NaN scores come first.
+ *   scores_in / ids_in   the runs, one block per shard: run r of query q is
+ *                        [bases[r] + run_offsets[r][q], bases[r] + run_offsets[r][q+1])
+ *   bases [S] int64, run_offsets [S][nq+1] int64 (every run_offsets[r] starts at 0 and is non-decreasing)
+ *   out_offsets [nq+1] int64 = the per-query sum of the runs' lengths, from 0 to `total`
+ *   scratch_scores / scratch_ids [total]: the intermediate result of the ceil(log2 S) two-way merge passes; needed when
+ *                        S > 2 (may be NULL otherwise)
+ *   scores / ids [total] the merged CSR values.
+ * Checks the offsets on the device and synchronises `stream` before merging.  MEVI_ERR_INVALID for S < 1, S > 8 or
+ * inconsistent offsets.                                                                                              */
+int mevi_merge_sorted_runs(mevi_ctx* ctx, const float* scores_in, const int64_t* ids_in, int S, int nq,
+                           const int64_t* bases, const int64_t* run_offsets, const int64_t* out_offsets, int64_t total,
+                           float* scratch_scores, int64_t* scratch_ids, float* scores, int64_t* ids, void* stream);
+
 /* ---- dense scorer -------------------------------------------------------- *
  * replaces: MEVI/document_encoder.py:128-132 compute_similarity(bmm=False):
  * out[nq, n] = Q[nq,d] . P[n,d]^T in fp32 (exact FMA accumulation).            */

@@ -64,6 +64,7 @@ SYMBOLS = {
     "mevi_flat_index_search": (_i, [_vp, _vp, _vp, _i, _i, _i64, _i, _vp, _vp, _vp]),
     "mevi_flat_index_destroy": (None, [_vp, _vp]),
     "mevi_topk_merge": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "mevi_merge_sorted_runs": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "mevi_dense_scores": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _vp]),
     "mevi_ensemble_cluster_ranks": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i64, _i, _vp, _i, _vp, _vp, _vp]),
     "mevi_ensemble_fuse": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _d, _d, _d, _i, _vp, _vp, _vp, _vp]),
@@ -717,6 +718,29 @@ class Context:
         ids = torch.empty((nq, k), dtype=torch.int64, device=s.device)
         with torch.cuda.device(self.device):
             self._check(self.lib.mevi_topk_merge(self.handle, _ptr(s), _ptr(i), S, nq, k, _ptr(scores), _ptr(ids), self._stream()))
+        return scores, ids
+
+    def merge_sorted_runs(self, scores_in, ids_in, bases, run_offsets, out_offsets):
+        """S runs per query, each sorted by (score desc, id asc): run r of query q is
+        [bases[r] + run_offsets[r, q], bases[r] + run_offsets[r, q+1]) of scores_in / ids_in  ->  the merged CSR values
+        (scores fp32 [total], ids int64 [total]) of out_offsets [nq+1].  One host sync (total, the offsets check)."""
+        import torch
+
+        s = self._dev(scores_in, torch.float32, "scores_in")
+        i = self._dev(ids_in, torch.int64, "ids_in")
+        b = self._dev(bases, torch.int64, "bases")
+        ro = self._dev(run_offsets, torch.int64, "run_offsets")
+        oo = self._dev(out_offsets, torch.int64, "out_offsets")
+        S, nq1 = ro.shape
+        if b.numel() != S or oo.numel() != nq1:
+            raise MeviError(f"bases [{b.numel()}] and out_offsets [{oo.numel()}] must match run_offsets [{S}, {nq1}]")
+        total = int(oo[-1].item())
+        scores = torch.empty(max(total, 0), dtype=torch.float32, device=s.device)
+        ids = torch.empty(max(total, 0), dtype=torch.int64, device=s.device)
+        tmp_s, tmp_i = (torch.empty_like(scores), torch.empty_like(ids)) if S > 2 else (None, None)
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mevi_merge_sorted_runs(self.handle, _ptr(s), _ptr(i), S, nq1 - 1, _ptr(b), _ptr(ro), _ptr(oo),
+                                                        total, _ptr(tmp_s), _ptr(tmp_i), _ptr(scores), _ptr(ids), self._stream()))
         return scores, ids
 
     def dense_scores(self, Q, P):

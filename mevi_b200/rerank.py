@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .dist_utils import all_gather_stack, dist_on, rank_world, shard_bounds
+from .dist_utils import all_gather_stack, all_gather_varlen, dist_on, rank_world, shard_bounds
 
 
 class ClusterIndex:
@@ -411,25 +411,41 @@ def _rerank_all(self, query_embedding, dec, multiclus_score_aggr: Optional[str] 
     under several of the query's leaves appears once, with its scores added or maximised (`np.unique` + loop there).
     Scores come from `mevi_cluster_rerank_all` (dense scorer's summation order, bit-equal to the top-k paths); the
     sort is a segmented device sort, ties ordered by ascending doc id (the reference's CUDA `torch.sort` leaves tie
-    order unspecified).  `--knn_topk_by_step` (3986-3989, a running top-pool_size) is `rerank(topk=pool_size)`."""
+    order unspecified).  `--knn_topk_by_step` (3986-3989, a running top-pool_size) is `rerank(topk=pool_size)`.
+    A leaf-partitioned shard (index.doc_ids set) maps its rows to document ids before the sort, so ties are ordered by
+    the document id.
+    With torch.distributed initialised the documents are sharded: every rank sorts its own candidates as above, the
+    per-rank CSRs are all-gathered and `mevi_merge_sorted_runs` merges the sorted runs, so every rank returns the whole
+    corpus's answer - bit-identical to the single-GPU call on the whole index: a candidate's score is computed from the
+    same row in the same order on whichever rank owns it, and (score, id) orders the candidates of different ranks
+    totally.  With 'add' and a document under c >= 3 of the query's leaves the single-GPU fold order is unspecified
+    (scatter_add_), so such scores agree within that rounding.  A multi-cluster call on a leaf-partitioned shard raises
+    NotImplementedError (a document's other leaves can live on other ranks); at most 8 ranks.  Extra device memory per
+    rank: the gathered runs and the output, 12 bytes per candidate of the whole corpus each, plus one more such buffer
+    with more than 2 ranks (the merge passes' intermediate)."""
     if not self.leaf_ordered:
         raise ValueError("rerank_all needs the leaf-ordered layout")
-    if dist_on():
-        raise NotImplementedError("rerank_all under torch.distributed: run it per shard and merge the sorted lists")
-    if self.index.doc_ids is not None:
-        raise NotImplementedError("rerank_all on a leaf-partitioned shard")
+    if multiclus_score_aggr is not None and multiclus_score_aggr not in ("add", "max"):
+        raise ValueError("multiclus_score_aggr must be 'add' or 'max' (main_models.py:4002-4009)")
+    idx = self.index
+    if multiclus_score_aggr is not None and idx.doc_ids is not None:
+        raise NotImplementedError("multi-cluster rerank_all on a leaf-partitioned shard: a document's other leaves can "
+                                  "live on other ranks")
+    world = rank_world()[1]
+    if world > 8:
+        raise NotImplementedError(f"rerank_all under torch.distributed merges at most 8 ranks (world size {world})")
     dev = self.D.device
     if not isinstance(query_embedding, torch.Tensor):
         query_embedding = torch.from_numpy(np.ascontiguousarray(query_embedding, dtype=np.float32))
     Q = query_embedding.to(device=dev, dtype=torch.float32).contiguous()
-    ql = self.index.lookup(dec)
-    offsets, scores, ids, _ = self.ctx.cluster_rerank_all(Q, self.D, self.index.leaf_offsets, self.index.leaf_docids, ql,
-                                                          id_base=self.index.id_base)
+    ql = idx.lookup(dec)
+    offsets, scores, ids, _ = self.ctx.cluster_rerank_all(Q, self.D, idx.leaf_offsets, idx.leaf_docids, ql,
+                                                          id_base=idx.id_base)
+    if idx.doc_ids is not None:  # leaf-partitioned shard: local rows -> document ids (id_base is 0 there)
+        ids = idx.doc_ids[ids]
     nq = Q.shape[0]
     seg = torch.repeat_interleave(torch.arange(nq, device=dev), offsets[1:] - offsets[:-1])
     if multiclus_score_aggr is not None:
-        if multiclus_score_aggr not in ("add", "max"):
-            raise ValueError("multiclus_score_aggr must be 'add' or 'max' (main_models.py:4002-4009)")
         span = int(ids.max().item()) + 1 if ids.numel() else 1
         key, inv = torch.unique(seg * span + ids, return_inverse=True)
         agg = torch.zeros(key.numel(), dtype=torch.float32, device=dev)
@@ -445,7 +461,21 @@ def _rerank_all(self, query_embedding, dec, multiclus_score_aggr: Optional[str] 
     order = torch.argsort(ids, stable=True)
     order = order[torch.argsort(scores[order], descending=True, stable=True)]
     order = order[torch.argsort(seg[order], stable=True)]
-    return offsets, ids[order], scores[order]
+    ids, scores = ids[order], scores[order]
+    if not dist_on():
+        return offsets, ids, scores
+    del order, seg
+    # every rank's sorted CSR to every rank (one block per rank), then one merge of the sorted runs
+    run_offsets = all_gather_stack(offsets)
+    gathered_scores = all_gather_varlen(scores)
+    del scores
+    gathered_ids = all_gather_varlen(ids)
+    del ids
+    run_len = run_offsets[:, -1]
+    bases = torch.cumsum(run_len, 0) - run_len
+    out_offsets = run_offsets.sum(0)
+    scores, ids = self.ctx.merge_sorted_runs(gathered_scores, gathered_ids, bases, run_offsets, out_offsets)
+    return out_offsets, ids, scores
 
 
 def hn_lines_all(texts: Sequence[str], offsets, ids, scores, save_hard_neg: Optional[int] = None,
