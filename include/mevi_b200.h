@@ -252,6 +252,27 @@ int mevi_cluster_rerank_all(mevi_ctx* ctx, const float* Q, int nq, const float* 
                             const int32_t* query_leaves, int L, int64_t id_base, const int64_t* out_offsets, float* scores,
                             int64_t* ids, int32_t* n_candidates, void* stream);
 
+/* The same call, same arguments, same outputs byte for byte (scores, ids, n_candidates), with every leaf's rows read
+ * once for all the queries that chose it: work items of one tile of <= 128 rows of a leaf x up to 256 of the leaf's
+ * (query, position) pairs, planned on the device inside the call (one host synchronisation).  The fp32 scores follow
+ * the streaming kernel's summation order exactly (the lane partials and its shuffle tree, evaluated as a pairwise
+ * sum in bit-reversed lane order), so no fp16 image is needed.  Scratch: about 28 bytes per (query, position) pair
+ * plus 24 bytes per leaf.                                                                                           */
+int mevi_cluster_rerank_all_grouped(mevi_ctx* ctx, const float* Q, int nq, const float* D_leaf, int64_t n, int d,
+                                    const int64_t* leaf_offsets, int64_t n_leaves, const int32_t* leaf_docids,
+                                    const int32_t* query_leaves, int L, int64_t id_base, const int64_t* out_offsets,
+                                    float* scores, int64_t* ids, int32_t* n_candidates, void* stream);
+
+/* Sorts every query's segment [offsets[q], offsets[q+1]) of (scores, ids) by score descending, then id ascending:
+ * -0.0 and +0.0 compare equal, NaN comes first, every element keeps its score bits.  This is the order of three stable
+ * torch.argsort passes (id, score descending, query) on the device.  offsets [nq+1] int64 device; the outputs may be
+ * the inputs.  Every id must lie in [0, 2^32) (MEVI_ERR_INVALID otherwise) and no query may hold 2^31 candidates or
+ * more.  Whole queries are sorted in chunks of at most 2^28 candidates (or one larger query), so totals above 2^31
+ * work.  Extra device memory: 24 bytes per candidate of the largest chunk (at most 6 GiB below 2^28) plus cub's
+ * temporary storage, kept in the context's scratch.  Two host synchronisations (offsets, id check).              */
+int mevi_sort_candidates(mevi_ctx* ctx, int nq, const int64_t* offsets, const float* scores_in, const int64_t* ids_in,
+                         float* scores_out, int64_t* ids_out, void* stream);
+
 /* ---- cluster-restricted re-rank as leaf-grouped GEMMs (tensor cores) ------ *
  * replaces: the same loop, MEVI/main_models.py:3915-4014.  A leaf selected by many queries is read ONCE and
  * scored against all of them: per leaf a [documents of the leaf] x [queries that chose it] fp16 tcgen05 GEMM whose

@@ -48,6 +48,9 @@ SYMBOLS = {
                                            _vp, _vp]),
     "mevi_cluster_rerank_prefix": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _i64, _vp, _vp, _i, _i, _i64, _vp, _vp, _vp, _vp]),
     "mevi_cluster_rerank_all": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _i64, _vp, _vp, _i, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "mevi_cluster_rerank_all_grouped": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _i64, _vp, _vp, _i, _i64, _vp, _vp, _vp, _vp,
+                                             _vp]),
+    "mevi_sort_candidates": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mevi_rerank_grouped_image": (_i, [_vp, _vp, _i64, _i, _vp, _i64, _vp, C.POINTER(_f), C.POINTER(_f), _vp]),
     "mevi_rerank_grouped_begin": (_i, [_vp, _vp, _i, _i, _f, _f, _vp, _vp]),
     "mevi_rerank_grouped_round": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _i, _i, _vp]),
@@ -475,9 +478,11 @@ class Context:
                 int(id_base), _ptr(scores), _ptr(ids), _ptr(ncand), self._stream()))
         return scores, ids, ncand
 
-    def cluster_rerank_all(self, Q, D_leaf, leaf_offsets, leaf_docids, query_leaves, id_base=0):
+    def cluster_rerank_all(self, Q, D_leaf, leaf_offsets, leaf_docids, query_leaves, id_base=0, grouped=False):
         """Scores of ALL candidates of every query, in the reference's concatenation order (unsorted):
-        -> (offsets int64 [nq+1], scores fp32 [total], ids int64 [total], n_candidates int32 [nq])."""
+        -> (offsets int64 [nq+1], scores fp32 [total], ids int64 [total], n_candidates int32 [nq]).
+        grouped=True: mevi_cluster_rerank_all_grouped (every leaf read once for all the queries that chose it), the same
+        arrays byte for byte."""
         import torch
 
         Q = self._dev(Q, torch.float32, "Q")
@@ -497,10 +502,36 @@ class Context:
         if total == 0:  # no query has a candidate (all its leaves are empty): nothing to score
             return offsets, scores, ids, ncand
         with torch.cuda.device(self.device):
-            self._check(self.lib.mevi_cluster_rerank_all(self.handle, _ptr(Q), nq, _ptr(D), D.shape[0], d, _ptr(lo), lo.numel() - 1,
-                                                         _ptr(ld), _ptr(ql), ql.shape[1], int(id_base), _ptr(offsets), _ptr(scores),
-                                                         _ptr(ids), _ptr(ncand), self._stream()))
+            fn = self.lib.mevi_cluster_rerank_all_grouped if grouped else self.lib.mevi_cluster_rerank_all
+            self._check(fn(self.handle, _ptr(Q), nq, _ptr(D), D.shape[0], d, _ptr(lo), lo.numel() - 1, _ptr(ld), _ptr(ql), ql.shape[1],
+                           int(id_base), _ptr(offsets), _ptr(scores), _ptr(ids), _ptr(ncand), self._stream()))
         return offsets, scores, ids, ncand
+
+    def cluster_rerank_all_grouped(self, Q, D_leaf, leaf_offsets, leaf_docids, query_leaves, id_base=0):
+        """cluster_rerank_all through mevi_cluster_rerank_all_grouped: the same four tensors, bit for bit."""
+        return self.cluster_rerank_all(Q, D_leaf, leaf_offsets, leaf_docids, query_leaves, id_base=id_base, grouped=True)
+
+    def sort_candidates(self, offsets, scores, ids, out=None):
+        """Every query's segment [offsets[q], offsets[q+1]) sorted by (score desc, id asc), -0.0 == +0.0, NaN first, score
+        bits kept: the order of three stable torch.argsort passes.  ids must lie in [0, 2^32).  -> (scores, ids); with
+        out=(scores_out, ids_out) the result goes there (it may be (scores, ids) themselves: sorted in place)."""
+        import torch
+
+        oo = self._dev(offsets, torch.int64, "offsets")
+        s = self._dev(scores, torch.float32, "scores")
+        i = self._dev(ids, torch.int64, "ids")
+        if s.numel() != i.numel():
+            raise MeviError(f"scores [{s.numel()}] and ids [{i.numel()}] differ in length")
+        if out is None:
+            out = (torch.empty_like(s), torch.empty_like(i))
+        so = self._dev(out[0], torch.float32, "scores_out")
+        io = self._dev(out[1], torch.int64, "ids_out")
+        if so.numel() != s.numel() or io.numel() != i.numel():
+            raise MeviError("outputs must match the inputs' length")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.mevi_sort_candidates(self.handle, oo.numel() - 1, _ptr(oo), _ptr(s), _ptr(i), _ptr(so), _ptr(io),
+                                                      self._stream()))
+        return so, io
 
     # ---- grouped (tensor-core) re-rank ------------------------------------------
     def cluster_rerank_prefix(self, Q, D_leaf, leaf_offsets, leaf_docids, query_leaves, k, max_rows):

@@ -29,6 +29,8 @@ enum WsSlot {
   WS_FLAT_IMAGE,    // one-shot flat search: fp16 image of the documents (+ its metadata)
   WS_GR_PLAN,       // grouped re-rank: device-side round plan (counts, scans, arrival numbers)
   WS_GR_MC,         // grouped re-rank of a multi-cluster index: per-query leaf tables, prefilter factors, margins
+  WS_RA_PLAN,       // grouped rerank_all: pairs by leaf, work-item scan
+  WS_RA_SORT,       // candidate sort: keys, values (double buffered), chunk offsets
   WS_NUM
 };
 

@@ -245,6 +245,9 @@ class ClusterReranker:
 
     AUTO_MIN_DOCS = 1 << 18         # mode='auto': corpora below this stay on the streaming kernel (no tile image)
     AUTO_QUERIES_PER_LEAF = 4       # mode='auto': grouped path when nq*L >= this many (query, leaf) pairs per leaf
+    AUTO_ALL_QUERIES_PER_LEAF = 0.25  # rerank_all, mode='auto': grouped scorer from this many (query, leaf) pairs per
+                                      # leaf.  Scoring at L = 10, 8.8 M x 768 (B200, 1,000 W): 0.12 pairs per leaf
+                                      # 4.3 ms stream / 4.8 ms grouped, 0.24: 7.8 / 7.5, 0.49: 14.7 / 10.2, 3.0: 75 / 23
     BOOTSTRAP_ROWS = 3072           # rows of the threshold-free first round per query (all appended: must fit the buffers)
     BOOTSTRAP_MIN = 2048            # fewer bootstrap rows than this: first threshold from the streaming kernel instead ...
     PASS_BUDGET = 6144              # ... unless the query has so few candidates that its sample's k-th best lets fewer than
@@ -409,9 +412,12 @@ def _rerank_all(self, query_embedding, dec, multiclus_score_aggr: Optional[str] 
         -> (offsets int64 [nq+1], ids int64 [total], scores fp32 [total]) on the device.
     `multiclus_score_aggr` in ('add', 'max') is the `--doc_multiclus > 1` aggregation of 3998-4011: a document listed
     under several of the query's leaves appears once, with its scores added or maximised (`np.unique` + loop there).
-    Scores come from `mevi_cluster_rerank_all` (dense scorer's summation order, bit-equal to the top-k paths); the
-    sort is a segmented device sort, ties ordered by ascending doc id (the reference's CUDA `torch.sort` leaves tie
-    order unspecified).  `--knn_topk_by_step` (3986-3989, a running top-pool_size) is `rerank(topk=pool_size)`.
+    Scores come from `mevi_cluster_rerank_all` (mode "stream": one pass over every query's candidates) or
+    `mevi_cluster_rerank_all_grouped` (mode "grouped": every leaf read once for all the queries that chose it; "auto"
+    takes it with at least AUTO_ALL_QUERIES_PER_LEAF (query, leaf) pairs per leaf of the index); both give the dense
+    scorer's summation order bit for bit (equal to the top-k paths), and `last_path` says which ran ("grouped-all" /
+    "stream-all").  The sort is `mevi_sort_candidates`, a segmented device sort (sort_candidates_torch restates it),
+    ties ordered by ascending doc id (the reference's CUDA `torch.sort` leaves tie order unspecified).  `--knn_topk_by_step` (3986-3989, a running top-pool_size) is `rerank(topk=pool_size)`.
     A leaf-partitioned shard (index.doc_ids set) maps its rows to document ids before the sort, so ties are ordered by
     the document id.
     With torch.distributed initialised the documents are sharded: every rank sorts its own candidates as above, the
@@ -439,13 +445,23 @@ def _rerank_all(self, query_embedding, dec, multiclus_score_aggr: Optional[str] 
         query_embedding = torch.from_numpy(np.ascontiguousarray(query_embedding, dtype=np.float32))
     Q = query_embedding.to(device=dev, dtype=torch.float32).contiguous()
     ql = idx.lookup(dec)
-    offsets, scores, ids, _ = self.ctx.cluster_rerank_all(Q, self.D, idx.leaf_offsets, idx.leaf_docids, ql,
-                                                          id_base=idx.id_base)
+    on_device = self.D.is_cuda
+    grouped = False
+    if on_device:  # the scorer: every leaf read once for all its queries, or one pass per query (the same bits)
+        grouped = self.mode == "grouped" or (
+            self.mode == "auto" and ql.numel() >= self.AUTO_ALL_QUERIES_PER_LEAF * max(1, idx.n_leaves))
+        self.last_path = "grouped-all" if grouped else "stream-all"
+        offsets, scores, ids, _ = self.ctx.cluster_rerank_all(Q, self.D, idx.leaf_offsets, idx.leaf_docids, ql,
+                                                              id_base=idx.id_base, grouped=grouped)
+    else:
+        offsets, scores, ids, _ = self.ctx.cluster_rerank_all(Q, self.D, idx.leaf_offsets, idx.leaf_docids, ql,
+                                                              id_base=idx.id_base)
     if idx.doc_ids is not None:  # leaf-partitioned shard: local rows -> document ids (id_base is 0 there)
         ids = idx.doc_ids[ids]
     nq = Q.shape[0]
-    seg = torch.repeat_interleave(torch.arange(nq, device=dev), offsets[1:] - offsets[:-1])
+    seg = None
     if multiclus_score_aggr is not None:
+        seg = torch.repeat_interleave(torch.arange(nq, device=dev), offsets[1:] - offsets[:-1])
         span = int(ids.max().item()) + 1 if ids.numel() else 1
         key, inv = torch.unique(seg * span + ids, return_inverse=True)
         agg = torch.zeros(key.numel(), dtype=torch.float32, device=dev)
@@ -457,14 +473,13 @@ def _rerank_all(self, query_embedding, dec, multiclus_score_aggr: Optional[str] 
         counts = torch.bincount(seg, minlength=nq)
         offsets = torch.zeros(nq + 1, dtype=torch.int64, device=dev)
         torch.cumsum(counts, 0, out=offsets[1:])
-    # segmented sort: (query asc, score desc, id asc) through three stable passes, least significant key first
-    order = torch.argsort(ids, stable=True)
-    order = order[torch.argsort(scores[order], descending=True, stable=True)]
-    order = order[torch.argsort(seg[order], stable=True)]
-    ids, scores = ids[order], scores[order]
+    if on_device:  # mevi_sort_candidates, in place
+        scores, ids = self.ctx.sort_candidates(offsets, scores, ids, out=(scores, ids))
+    else:
+        scores, ids = sort_candidates_torch(offsets, scores, ids)
+    del seg
     if not dist_on():
         return offsets, ids, scores
-    del order, seg
     # every rank's sorted CSR to every rank (one block per rank), then one merge of the sorted runs
     run_offsets = all_gather_stack(offsets)
     gathered_scores = all_gather_varlen(scores)
@@ -476,6 +491,18 @@ def _rerank_all(self, query_embedding, dec, multiclus_score_aggr: Optional[str] 
     out_offsets = run_offsets.sum(0)
     scores, ids = self.ctx.merge_sorted_runs(gathered_scores, gathered_ids, bases, run_offsets, out_offsets)
     return out_offsets, ids, scores
+
+
+def sort_candidates_torch(offsets, scores, ids):
+    """Every query's segment of a CSR sorted by (score desc, id asc) through three stable torch passes, least significant
+    key first: the restatement of `mevi_sort_candidates` (Context.sort_candidates), and rerank_all's sort on CPU tensors.
+    -> (scores, ids)."""
+    nq = offsets.numel() - 1
+    seg = torch.repeat_interleave(torch.arange(nq, device=offsets.device), offsets[1:] - offsets[:-1])
+    order = torch.argsort(ids, stable=True)
+    order = order[torch.argsort(scores[order], descending=True, stable=True)]
+    order = order[torch.argsort(seg[order], stable=True)]
+    return scores[order], ids[order]
 
 
 def hn_lines_all(texts: Sequence[str], offsets, ids, scores, save_hard_neg: Optional[int] = None,

@@ -12,7 +12,14 @@ each timed with CUDA events after two warm-up calls (medians of --reps calls; th
 and the whole `rerank_all` call.  Also: peak device memory per rank over one whole call, and a SHA-256 of the result
 (offsets, ids, score bits).  With --ref FILE a world-size-1 run writes its digests there and a larger run compares its
 own against them (bit-equality flag).  Prints one JSON line (rank 0).
-Usage: torchrun --nproc-per-node N tools/dist_rerank_all_time.py [--reps 3] [--leaves 10,100] [--ref FILE]"""
+On one GPU the same run also times, next to the above, the leaf-grouped scorer (mevi_cluster_rerank_all_grouped:
+score_grouped_ms, its TFLOP/s from 2 d per candidate against the fp32 FMA bound of 148 SMs x 128 lanes x 2 x 1,965 MHz,
+the row bytes each scorer requests), the device sort (mevi_sort_candidates: sort_device_ms, next to the torch sort),
+the whole call on each path (rerank_all_stream_ms, rerank_all_grouped_ms), peak extra memory of each whole call
+(torch allocations + growth of the library's scratch) and SHA-256 digests of both paths' results, which must agree.
+--sweep Q1,Q2,...: also time both scorers at L = 10 on the first Qi queries (the pairs-per-leaf threshold of
+mode="auto").
+Usage: torchrun --nproc-per-node N tools/dist_rerank_all_time.py [--reps 3] [--leaves 10,100] [--ref FILE] [--out FILE]"""
 import argparse
 import hashlib
 import json
@@ -25,11 +32,13 @@ import torch.distributed as dist
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import mevi_b200  # noqa: E402
+import mevi_b200.rerank  # noqa: E402
 from mevi_b200.dist_utils import all_gather_stack, all_gather_varlen, dist_on, shard_bounds  # noqa: E402
 from mevi_b200.pq import ProductQuantization  # noqa: E402
 from mevi_b200.rerank import ClusterIndex, ClusterReranker  # noqa: E402
 
 HBM_PEAK = 7.7e12  # bytes/s, B200 data sheet (one GPU)
+FP32_FMA_PEAK = 148 * 128 * 2 * 1.965e9  # FLOP/s: 148 SMs x 128 fp32 lanes x 2 x 1,965 MHz boost clock
 
 
 def digest(off, ids, sc):
@@ -55,6 +64,73 @@ def median_ms(fn, reps, sync):
     return sorted(ts)[len(ts) // 2]
 
 
+def extra_memory(fn, sync, dev):
+    """(result, GiB): peak device memory of one call above what was allocated before it - torch's allocations plus the
+    growth of the library's scratch (cudaMalloc outside torch, seen as free memory lost beyond torch's reserve)."""
+    sync()
+    torch.cuda.empty_cache()
+    free0, res0 = torch.cuda.mem_get_info(dev)[0], torch.cuda.memory_reserved(dev)
+    torch.cuda.reset_peak_memory_stats(dev)
+    base = torch.cuda.memory_allocated(dev)
+    out = fn()
+    sync()
+    peak = torch.cuda.max_memory_allocated(dev) - base
+    torch.cuda.empty_cache()
+    lib = max(0, (free0 - torch.cuda.mem_get_info(dev)[0]) - (torch.cuda.memory_reserved(dev) - res0))
+    return out, round((peak + lib) / 2**30, 2)
+
+
+def grouped_times(ctx, rr, index, Q, dec, L, reps, sync, dev):
+    """The leaf-grouped scorer and the device sort next to the streaming scorer and the torch sort (one GPU)."""
+    d = rr.D.shape[1]
+    rg = mevi_b200.rerank.ClusterReranker(None, index, mode="grouped", D_leaf=rr.D)
+    ql = index.lookup(dec)
+    st = {}
+    t = {}
+    t["score_grouped_ms"] = median_ms(lambda: st.__setitem__("g", ctx.cluster_rerank_all_grouped(
+        Q, rr.D, index.leaf_offsets, index.leaf_docids, ql, id_base=index.id_base)), reps, sync)
+    off, sc, ids, _ = st.pop("g")
+    out = (torch.empty_like(sc), torch.empty_like(ids))
+    t["sort_device_ms"] = median_ms(lambda: ctx.sort_candidates(off, sc, ids, out=out), reps, sync)
+    del out, sc, ids
+    cand = int(off[-1])
+    sizes = index.leaf_offsets[1:] - index.leaf_offsets[:-1]
+    valid = ql >= 0
+    pairs = torch.bincount(ql[valid].long(), minlength=sizes.numel())
+    chunks = (pairs + 255) // 256  # an item meets up to 256 of its leaf's pairs
+    t["grouped_tflops"] = round(2 * d * cand / (t["score_grouped_ms"] * 1e-3) / 1e12, 2)
+    t["grouped_share_of_fp32_fma_peak"] = round(2 * d * cand / (t["score_grouped_ms"] * 1e-3) / FP32_FMA_PEAK, 3)
+    t["row_bytes_stream_gb"] = round(4 * d * cand / 1e9, 1)
+    t["row_bytes_grouped_items_gb"] = round(4 * d * int((sizes * chunks).sum()) / 1e9, 1)
+    t["row_bytes_distinct_gb"] = round(4 * d * int(sizes[pairs > 0].sum()) / 1e9, 1)
+    t["pairs_per_leaf"] = round(ql.numel() / max(1, index.n_leaves), 2)
+    t["rerank_all_stream_ms"] = median_ms(lambda: rr.rerank_all(Q, dec), reps, sync)
+    t["rerank_all_grouped_ms"] = median_ms(lambda: rg.rerank_all(Q, dec), reps, sync)
+    (o1, i1, s1), t["peak_extra_gib_stream"] = extra_memory(lambda: rr.rerank_all(Q, dec), sync, dev)
+    d_stream = digest(o1, i1, s1)
+    del o1, i1, s1
+    (o2, i2, s2), t["peak_extra_gib_grouped"] = extra_memory(lambda: rg.rerank_all(Q, dec), sync, dev)
+    t["path_grouped"] = rg.last_path
+    d_grouped = digest(o2, i2, s2)
+    del o2, i2, s2
+    t["digest_stream"], t["digest_grouped"] = d_stream, d_grouped
+    t["digests_equal"] = d_stream == d_grouped
+    return {k: (round(v, 2) if isinstance(v, float) else v) for k, v in t.items()}
+
+
+def sweep(ctx, rr, index, Q, dec, counts, reps, sync):
+    """Both scorers on the first nq queries: where the grouped one starts to win (mode="auto")."""
+    out = []
+    for nq in counts:
+        q, ql = Q[:nq].contiguous(), index.lookup(dec[:nq])
+        a = (q, rr.D, index.leaf_offsets, index.leaf_docids, ql)
+        ms_s = median_ms(lambda: ctx.cluster_rerank_all(*a, id_base=index.id_base), reps, sync)
+        ms_g = median_ms(lambda: ctx.cluster_rerank_all_grouped(*a, id_base=index.id_base), reps, sync)
+        out.append(dict(queries=nq, pairs_per_leaf=round(ql.numel() / max(1, index.n_leaves), 3), score_stream_ms=round(ms_s, 3),
+                        score_grouped_ms=round(ms_g, 3)))
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=3)
@@ -62,6 +138,8 @@ def main():
     ap.add_argument("--docs", type=int, default=8841823)
     ap.add_argument("--queries", type=int, default=6980)
     ap.add_argument("--ref", default=None)
+    ap.add_argument("--sweep", default="")
+    ap.add_argument("--out", default=None)
     args = ap.parse_args()
     local = int(os.environ.get("LOCAL_RANK", 0))
     dev = torch.device("cuda", local)
@@ -165,9 +243,18 @@ def main():
             t["bit_equal_to_n1"] = ref.get(f"L{L}") == digests[f"L{L}"]
         peaks = all_gather_stack(torch.tensor([t["peak_extra_gib_per_rank"]], device=dev)).flatten().tolist()
         t["peak_extra_gib_all_ranks"] = peaks
+        del off, ids, sc
+        if world == 1:
+            t.update(grouped_times(ctx, rr, index, Q, dec, L, args.reps, sync, dev))
         res[f"L{L}"] = {k: (round(v, 2) if isinstance(v, float) else v) for k, v in t.items()}
-        del off, ids, sc, dec
+        del dec
         torch.cuda.empty_cache()
+    if world == 1 and args.sweep:
+        dec = torch.cat([pq.beam_search(Q[a : a + 1024], 10) for a in range(0, Q.shape[0], 1024)])
+        res["auto_sweep_L10"] = sweep(ctx, rr, index, Q, dec, [int(v) for v in args.sweep.split(",")], args.reps, sync)
+    if rank == 0 and args.out:
+        with open(args.out, "w") as fw:
+            json.dump(res, fw, indent=1)
     if rank == 0:
         if args.ref and world == 1:
             with open(args.ref, "w") as fw:
